@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- hands/s of the fused geometry step (MANO + LBS + PCL + projection, fwd+bwd) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--samples S]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--samples S] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[3], the one the metric is quoted on, as one GPU's shard):
@@ -246,6 +246,8 @@ def run_ours(args, rank, world, local_rank):
     launches = _lib.launch_count() - l0 + graph_launches * args.steps   # replays launch the captured kernels without host calls
     elapsed = e0.elapsed_time(e1) * 1e-3
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:   # before the legs below reuse the step's buffers
+        dump_outputs(step, args.dump_outputs)
     if world > 1:
         t = torch.tensor([elapsed], device=dev, dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -396,6 +398,38 @@ def run_ours(args, rank, world, local_rank):
     print(json.dumps(line), flush=True)
 
 
+DUMP_HAND_SAMPLES = 512    # samples whose per-hand outputs are written (40 KB per sample)
+DUMP_IMAGE_SAMPLES = 16    # samples whose crops and source-image gradient are written (1.8 MB per sample)
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(step, out_dir):
+    """Write what the last step left in its output buffers, i.e. what a caller of the step receives, as `out_dir/<name>.npy`
+    (float32), so that two builds can be compared output for output.  The whole output of an 8192-sample step is ~15 GB,
+    so a fixed sample of it is written, ~50 MB: the per-hand outputs of 512 samples and the crops and image gradients of
+    16 samples, both drawn by a seeded permutation of the sample index.  Crop rows are [sample][right, left]."""
+    import numpy as np
+
+    perm = torch.randperm(step.S, generator=torch.Generator().manual_seed(0))
+    hand_idx = perm[:DUMP_HAND_SAMPLES].sort().values.to(step.dev)
+    img_idx = perm[:DUMP_IMAGE_SAMPLES].sort().values.to(step.dev)
+    crop_idx = (img_idx[:, None] * step.hps + torch.arange(step.hps, device=step.dev)).flatten()
+    out = {
+        "crops": step.crops[crop_idx],
+        "g_img": step.g_img[img_idx],
+        "rot": step.rot.view(step.S, step.hps, 3, 3)[hand_idx],
+    }
+    for side, h in zip(("right", "left"), step.hands):
+        for key in ("vertices", "v3d", "joints3d", "j3d", "j2d", "cam_t", "g_rotmat", "g_betas", "g_cam"):
+            out[f"{side}_{key}"] = h[key][hand_idx]
+    out = {k: v.float().cpu().numpy() for k, v in out.items()}
+    total = sum(a.nbytes for a in out.values())
+    assert total <= DUMP_MAX_BYTES, total
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def L_c5(dev, world, rank, args):
     """C5: HaMeR-light MANO head training step with the parameter-gradient all-reduce (scripts/c5_hamer_head.py), both the
     read-out-sized (894 KB) and the decoder-head-sized (158 MB) gradient."""
@@ -537,7 +571,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="launch the step kernel by kernel instead of replaying its CUDA graph")
     ap.add_argument("--quick", action="store_true", help="skip the side legs (other configs, fp32-source e2e, CPU worker pool)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a fixed sample of the last timed step's outputs to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
