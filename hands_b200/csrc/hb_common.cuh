@@ -43,10 +43,6 @@ struct ManoConst {
   int tips[5];
 };
 
-// Scatter form of the transposed grid_sample (pcl_bwd_scatter_kernel): rolling window of source rows in shared memory.
-constexpr int PCL_SC_H = 32;        // window rows (power of two)
-constexpr int PCL_SC_MAXNP = 6;     // most row phases the kernel is willing to run (record slot 26 holds the count, 0 = not eligible)
-
 extern std::atomic<uint64_t> g_launches;
 void set_error(const char* fmt, ...);
 int check_launch(const char* what);

@@ -941,13 +941,8 @@ static bool use_tc() {
 
 // CTAs per (16-hand group, vertex slice) of the skinning kernels: the group's hands are split over two CTAs (shorter serial
 // chain per CTA, twice the CTAs in flight).  Measured fwd+bwd of one side, 1 vs 2: 1024 hands 162 -> 145 us, 2048 221 -> 207,
-// 4096 344 -> 337, 8192 626 -> 614.  HB_MANO_HSPLIT=1 restores one CTA per pair.
-static unsigned skin_hsplit(int B) {
-  (void)B;
-  static int forced = -1;
-  if (forced < 0) { const char* e = getenv("HB_MANO_HSPLIT"); forced = e ? atoi(e) : 0; }
-  return forced == 1 ? 1u : 2u;
-}
+// 4096 344 -> 337, 8192 626 -> 614.
+constexpr unsigned kSkinHsplit = 2;
 
 static const size_t kSkinFwdSmem = sizeof(float) * (FS * HBF + HBF * AS + HBF * 8 + HBF * XS);
 static const size_t kSkinFwdSmemTc = sizeof(float) * (HBF * AS + HBF * 8 + HBF * XS);
@@ -980,7 +975,7 @@ extern "C" int hb_mano_head_fwd(const hb_mano* h, const float* pose, int pose_fo
   rc = check_launch("mano_pose_fwd_kernel");
   if (rc) return rc;
   SkinFwdOut o{vertices, v3d_cam, joints3d, j3d_cam, j2d_norm};
-  dim3 grid((unsigned)ws_groups(B), NSLICE, skin_hsplit(B));
+  dim3 grid((unsigned)ws_groups(B), NSLICE, kSkinHsplit);
   if (tc) {
     rc = launch_blend_tc(fh, fl, h->c.Bhi, h->c.Blo, h->c.Vt, B, vpo, st);
     if (rc) return rc;
@@ -1023,7 +1018,7 @@ static int mano_head_bwd_impl(const hb_mano* h, const float* pose, int pose_form
     if (rc) return rc;
   }
   SkinBwdIn gi{g_vertices, g_v3d_cam, g_joints3d, g_j3d_cam, g_j2d_norm};
-  dim3 grid((unsigned)ws_groups(B), NSLICE, skin_hsplit(B));
+  dim3 grid((unsigned)ws_groups(B), NSLICE, kSkinHsplit);
   if (tc) {
     if (!reuse) {
       rc = launch_blend_tc(fh, fl, h->c.Bhi, h->c.Blo, h->c.Vt, B, vpo, st);

@@ -54,42 +54,6 @@ __host__ __device__ inline int pcl_homography64(const int32_t* bb, const float* 
   return s;
 }
 
-// Eligibility of a crop for the scatter form of the backward (pcl_bwd_scatter_kernel) and the number of row phases it
-// needs; 0 = not eligible (the gather kernel takes the image).  With (x, y)(u, v) = (N_x, N_y) / D, D = P6 u + P7 v + P8:
-//   dx/du = a(v) / D^2, dy/du = b(v) / D^2, dx/dv = c(u) / D^2, dy/dv = d(u) / D^2   with a, b, c, d LINEAR,
-// so over the unit square every partial derivative is bounded by the end values of its numerator over the corner values of
-// D (rigorous, a little loose).  Per grid step (1/(s-1)) the kernel needs:
-//   * x strictly increasing along a row by more than half a pixel per sample (at most two samples share a pixel column);
-//   * y increasing from row to row, and rows NP apart touching disjoint pixels wherever they are within two columns of
-//     each other:  NP yj_min - (2 + NP |xj|) / xi_min * |yi| >= 2  (mean-value bound on the displacement);
-//   * NP rows plus the drift of a row across the crop fit the window.
-__device__ int scatter_phases(const double* P, int s, int img_res) {
-  if (s < 2 || s > img_res) return 0;
-  double dmin = 1e300, dmax = -1e300;
-  for (int cy = 0; cy < 2; ++cy)
-    for (int cx = 0; cx < 2; ++cx) {
-      const double D = P[6] * cx + P[7] * cy + P[8] + 1e-8;
-      dmin = fmin(dmin, D); dmax = fmax(dmax, D);
-    }
-  if (!(dmin > 1e-9) || !(dmax < 1e300)) return 0;
-  const double du = 1.0 / (double)(s - 1);
-  const double lo2 = du / (dmax * dmax), hi2 = du / (dmin * dmin);
-  const double a0 = P[0] * P[8] - P[2] * P[6], a1 = a0 + (P[0] * P[7] - P[1] * P[6]);
-  const double b0 = P[3] * P[8] - P[5] * P[6], b1 = b0 + (P[3] * P[7] - P[4] * P[6]);
-  const double c0 = P[1] * P[8] - P[2] * P[7], c1 = c0 + (P[1] * P[6] - P[0] * P[7]);
-  const double d0 = P[4] * P[8] - P[5] * P[7], d1 = d0 + (P[4] * P[6] - P[3] * P[7]);
-  const double xi_min = fmin(a0, a1) * lo2;
-  const double yj_min = fmin(d0, d1) * lo2, yj_max = fmax(d0, d1) * hi2;
-  const double yi_abs = fmax(fabs(b0), fabs(b1)) * hi2, xj_abs = fmax(fabs(c0), fabs(c1)) * hi2;
-  if (!(xi_min > 0.55) || !(yj_min > 0.0)) return 0;
-  for (int np = 3; np <= PCL_SC_MAXNP; ++np) {
-    if (np * yj_min - (2.0 + np * xj_abs) / xi_min * yi_abs < 2.05) continue;
-    if (np * yj_max + (double)(s - 1) * yi_abs + 4.5 > (double)PCL_SC_H) return 0;
-    return np;
-  }
-  return 0;
-}
-
 __global__ void pcl_setup_kernel(const int32_t* __restrict__ bbox, const float* __restrict__ K, int n, int img_res,
                                  float* __restrict__ params, float* __restrict__ Rout) {
   const int q = blockIdx.x * blockDim.x + threadIdx.x;
@@ -135,7 +99,6 @@ __global__ void pcl_setup_kernel(const int32_t* __restrict__ bbox, const float* 
   rec[22] = __int_as_float(fx0); rec[23] = __int_as_float(fx1); rec[24] = __int_as_float(fy0); rec[25] = __int_as_float(fy1);
 #pragma unroll
   for (int k = 26; k < PF; ++k) rec[k] = 0.0f;
-  rec[26] = __int_as_float(scatter_phases(Pf, s, img_res));
   if (Rout) {
 #pragma unroll
     for (int k = 0; k < 9; ++k) Rout[(size_t)q * 9 + k] = (float)Rv[k];

@@ -12,7 +12,6 @@ through the C ABI on the current stream, with no allocation and no autograd book
 drop-ins in `hands_b200.functional` call the same entry points; this class only removes the per-call allocations.
 """
 import ctypes
-import os
 
 import torch
 
@@ -82,9 +81,9 @@ class GeometryStep:
             self.mano_ws_bytes = self.lib.hb_mano_workspace_bytes(S, 1)
             self.mano_ws = [torch.empty((self.mano_ws_bytes + 3) // 4, **f32) for _ in range(hands_per_sample)]
             self.mano_fwd_valid = [False] * hands_per_sample
-        # second stream for the left hand side of the fused step (HB_STEP_MANO_STREAMS=1: everything on one stream)
+        # second stream for the left hand side of the fused step
         self.mano_side_stream = None
-        if with_mano and hands_per_sample == 2 and os.environ.get("HB_STEP_MANO_STREAMS", "2") != "1":
+        if with_mano and hands_per_sample == 2:
             self.mano_side_stream = torch.cuda.Stream(device=self.dev)
 
     # ---- pieces (each enqueues on the CURRENT torch stream) ------------------------------------
@@ -147,7 +146,7 @@ class GeometryStep:
             if self.with_mano:
                 if self.with_pcl:
                     self.gather_pre_rot()
-                if self.hps == 2 and self.mano_side_stream is not None:
+                if self.mano_side_stream is not None:
                     # the two hand sides are independent (own constants, inputs, workspace): the left side runs on a forked
                     # stream, so its latency-bound kernels (pose, the tcgen05 contractions: at most one CTA per SM) share the
                     # GPU with the right side's skinning kernels; joined before the crop layer's backward.  Inside a capture

@@ -53,7 +53,7 @@ typedef struct hb_mano hb_mano; /* opaque: MANO constants of one hand side on on
 #define HB_ROT6D_COLS 1        /* src/models/hamer_light/geometry.py:47-62, src/models/handoccnet_light/mano_head.py:132-141: a1=x[0:3], a2=x[3:6], COLUMNS */
 #define HB_ROT6D_COLS_PAIRED 2 /* common/rot.py:367-381: a1=x[0,2,4], a2=x[1,3,5], COLUMNS */
 
-#define HB_VERSION 202 /* hb_version() of a matching binary */
+#define HB_VERSION 203 /* hb_version() of a matching binary */
 const char* hb_last_error_string(void);
 int hb_version(void);
 
@@ -223,12 +223,6 @@ int hb_pcl_fwd(const float* img, const float* params, int n_crops, int crops_per
  *   (bit-identical on > 99.9 % of the pixels, ~1.3x the instructions).  Environment HB_PCL_EXACT sets the initial value.
  *   Returns the previous setting.  Process-wide. */
 int hb_pcl_set_exact(int on);
-/* Backward of the resampling step for 3 x 224 x 224 images: 1 (default) = scatter form (pcl_bwd_scatter_kernel: the samples
- *   of an intermediate row, about one source pixel apart, are added into a rolling shared-memory window of source rows in a
- *   fixed order, no atomics); crops whose homography the setup kernel's bounds reject, other shapes, and 0 = gather form
- *   through per-pixel lists (pcl_bwd_img_kernel).  Both are bit-reproducible; they differ from each other by fp32 summation
- *   order.  Environment HB_PCL_SCATTER sets the initial value.  Returns the previous setting.  Process-wide. */
-int hb_pcl_set_scatter(int on);
 /* Same crop from the data loader's 8-bit image (n_crops/crops_per_img, C, R, R) uint8: x = (u/255 - mean[c]) / std[c]
  *   (torchvision Normalize as the reference applies it to the full image, src/datasets/hands_light_dataset.py:177-184)
  *   is fused into the gather, so the result equals hb_pcl_fwd on the normalised fp32 image while a quarter of the bytes

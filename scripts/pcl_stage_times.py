@@ -31,20 +31,8 @@ def main():
     st.pcl_backward()
     out = {"images": n,
            "fwd_us": cuda_time(st.pcl_forward),
-           "mid_us": cuda_time(lambda: st.pcl_backward_stage(1))}
-    # transposed grid_sample: scatter form (default) and gather form, same workspace contents
-    ref = None
-    for name, on in (("img_scatter_us", 1), ("img_gather_us", 0)):
-        prev = st.lib.hb_pcl_set_scatter(on)
-        out[name] = cuda_time(lambda: st.pcl_backward_stage(2))
-        g = st.g_img.clone()
-        st.lib.hb_pcl_set_scatter(prev)
-        if ref is None:
-            ref = g
-        else:
-            out["scatter_vs_gather_rel"] = float((ref - g).abs().max() / g.abs().max())
-    out["eligible_frac"] = float((st.params[:, 26].view(torch.int32) > 0).float().mean())
-    out["phases_hist"] = torch.bincount(st.params[:, 26].view(torch.int32).cpu(), minlength=7).tolist()
+           "mid_us": cuda_time(lambda: st.pcl_backward_stage(1)),
+           "img_us": cuda_time(lambda: st.pcl_backward_stage(2))}
     print(json.dumps(out))
 
 

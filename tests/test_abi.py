@@ -34,8 +34,8 @@ def test_workspace_sizes_and_argument_errors():
     lib = _lib.load()
     assert lib.hb_mano_workspace_bytes(0, 0) == 0
     assert lib.hb_mano_workspace_bytes(1024, 1) > lib.hb_mano_workspace_bytes(1024, 0) > 0
-    assert lib.hb_pcl_bwd_workspace_bytes(8, 2, 3, 224) == 8 * 4 * 224 * 224 * 4 + 4 * 16  # one float4 gradient per intermediate pixel + 16 B per image (fallback list)
-    assert lib.hb_pcl_bwd_workspace_bytes(2 * 8192, 2, 3, 224) == 2 * 4096 * 4 * 224 * 224 * 4 + 4096 * 16  # capped at 4096 images per chunk
+    assert lib.hb_pcl_bwd_workspace_bytes(8, 2, 3, 224) == 8 * 4 * 224 * 224 * 4  # one float4 gradient per intermediate pixel
+    assert lib.hb_pcl_bwd_workspace_bytes(2 * 8192, 2, 3, 224) == 2 * 4096 * 4 * 224 * 224 * 4  # capped at 4096 images per chunk
     # argument validation happens before any CUDA call, so it is testable without a GPU
     rc = lib.hb_mano_head_fwd(None, None, 1, None, None, None, None, None, 4, 224.0, 0.1, None, None, None, None, None, None, None, 0, None)
     assert rc == -1 and b"NULL" in lib.hb_last_error_string()
