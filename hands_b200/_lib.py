@@ -18,7 +18,6 @@ SYMBOLS = {
     "hb_mano_create": (ctypes.c_int, [ctypes.c_void_p] * 8 + [ctypes.c_int, ctypes.POINTER(ctypes.c_void_p)]),
     "hb_mano_destroy": (ctypes.c_int, [ctypes.c_void_p]),
     "hb_mano_workspace_bytes": (ctypes.c_size_t, [ctypes.c_int, ctypes.c_int]),
-    "hb_mano_set_tensor_core": (ctypes.c_int, [ctypes.c_int]),
     "hb_mano_head_fwd": (
         ctypes.c_int,
         [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,

@@ -8,7 +8,6 @@
 namespace hb {
 
 std::atomic<uint64_t> g_launches{0};
-int g_mano_tc = -1;   // -1: not decided yet (env HB_MANO_TC, default on)
 static thread_local char g_err[512] = "";
 
 void set_error(const char* fmt, ...) {
@@ -33,7 +32,6 @@ using namespace hb;
 
 extern "C" const char* hb_last_error_string(void) { return g_err; }
 extern "C" int hb_version(void) { return HB_VERSION; }
-extern "C" int hb_mano_set_tensor_core(int on) { const int prev = g_mano_tc; g_mano_tc = on ? 1 : 0; return prev; }
 extern "C" uint64_t hb_launch_count(void) { return g_launches.load(); }
 
 extern "C" int hb_mano_create(const float* v_template, const float* shapedirs, const float* posedirs, const float* J_regressor,
@@ -65,24 +63,17 @@ extern "C" int hb_mano_create(const float* v_template, const float* shapedirs, c
     c.tips[k] = tip_ids[k];
   }
   // host-side re-layout
-  const size_t nPk = (size_t)NP * 3 * VP, nPt = (size_t)3 * VP * FS, nVt = (size_t)3 * VP, nWt = (size_t)NJ * VP, nWv = (size_t)VP * NJ;
+  const size_t nVt = (size_t)3 * VP, nWt = (size_t)NJ * VP, nWv = (size_t)VP * NJ;
   const size_t nJt = NJ * 3, nJsd = NJ * 3 * NB, nPm = 48;
   const size_t nB = (size_t)10 * 19 * 240 * 8;   // tensor-core operand slabs
   const size_t nPs = (size_t)300 * 160 * 8;
   size_t off = 0;
   auto take = [&](size_t n) { size_t o = off; off += (n + 3) / 4 * 4; return o; };  // keep 16-byte alignment
-  const size_t oPk = take(nPk), oPt = take(nPt), oVt = take(nVt), oWt = take(nWt), oWv = take(nWv), oJt = take(nJt), oJsd = take(nJsd), oPm = take(nPm), oBh = take(nB), oBl = take(nB), oPh = take(nPs), oPl = take(nPs);
+  const size_t oVt = take(nVt), oWt = take(nWt), oWv = take(nWv), oJt = take(nJt), oJsd = take(nJsd), oPm = take(nPm), oBh = take(nB), oBl = take(nB), oPh = take(nPs), oPl = take(nPs);
   std::vector<float> hostbuf(off, 0.0f);
-  float* Pk = hostbuf.data() + oPk; float* Pt = hostbuf.data() + oPt; float* Vt = hostbuf.data() + oVt;
+  float* Vt = hostbuf.data() + oVt;
   float* Wt = hostbuf.data() + oWt; float* Wv = hostbuf.data() + oWv; float* Jt = hostbuf.data() + oJt;
   float* Jsd = hostbuf.data() + oJsd; float* Pm = hostbuf.data() + oPm;
-  for (int p = 0; p < NP; ++p)
-    for (int k = 0; k < 3; ++k)
-      for (int v = 0; v < NV; ++v) {
-        const float val = p < NPF ? posedirs[(size_t)p * (NV * 3) + 3 * v + k] : shapedirs[((size_t)v * 3 + k) * NB + (p - NPF)];
-        Pk[((size_t)p * 3 + k) * VP + v] = val;
-        Pt[((size_t)k * VP + v) * FS + p] = val;
-      }
   for (int v = 0; v < NV; ++v) {
     for (int k = 0; k < 3; ++k) Vt[(size_t)k * VP + v] = v_template[v * 3 + k];
     for (int j = 0; j < NJ; ++j) { Wt[(size_t)j * VP + v] = lbs_weights[v * NJ + j]; Wv[(size_t)v * NJ + j] = lbs_weights[v * NJ + j]; }
@@ -99,6 +90,10 @@ extern "C" int hb_mano_create(const float* v_template, const float* shapedirs, c
       }
     }
   for (int k = 0; k < 48; ++k) Pm[k] = pose_mean[k];
+  // stacked blendshape basis [posedirs; shapedirs^T]: row p < NP, coordinate k of vertex v < NV
+  auto basis = [&](int p, int k, int v) {
+    return p < NPF ? posedirs[(size_t)p * (NV * 3) + 3 * v + k] : shapedirs[((size_t)v * 3 + k) * NB + (p - NPF)];
+  };
   // tensor-core B operand: column c' = k*800 + v (coordinate-major), tile = c'/240, UMMA K-major no-swizzle slabs
   // [tile][k-step][k-half][row-group][row][4]; split into TF32 hi/lo parts
   {
@@ -110,7 +105,7 @@ extern "C" int hb_mano_create(const float* v_template, const float* shapedirs, c
           for (int kk = 0; kk < 8; ++kk) {
             const int cp = tile * 240 + n, pidx = ks * 8 + kk;
             const int k = cp / VP, v = cp % VP;
-            const float val = (pidx < NP && v < NV) ? Pk[((size_t)pidx * 3 + k) * VP + v] : 0.0f;
+            const float val = (pidx < NP && v < NV) ? basis(pidx, k, v) : 0.0f;
             const float hi = tf32_round(val), lo = tf32_round(val - hi);
             const size_t o = ((size_t)tile * 19 + ks) * 1920 + (size_t)(kk >> 2) * 960 + (n >> 3) * 32 + (n & 7) * 4 + (kk & 3);
             Bh[o] = hi; Bl[o] = lo;
@@ -123,7 +118,7 @@ extern "C" int hb_mano_create(const float* v_template, const float* shapedirs, c
         for (int kk = 0; kk < 8; ++kk) {
           const int cp = ks * 8 + kk;
           const int k = cp / VP, v = cp % VP;
-          const float val = (pidx < NP && v < NV) ? Pk[((size_t)pidx * 3 + k) * VP + v] : 0.0f;
+          const float val = (pidx < NP && v < NV) ? basis(pidx, k, v) : 0.0f;
           const float hi = tf32_round(val), lo = tf32_round(val - hi);
           const size_t o = (size_t)ks * 1280 + (size_t)(kk >> 2) * 640 + (pidx >> 3) * 32 + (pidx & 7) * 4 + (kk & 3);
           Ph[o] = hi; Pl[o] = lo;
@@ -143,7 +138,7 @@ extern "C" int hb_mano_create(const float* v_template, const float* shapedirs, c
     return (int)e;
   }
   const float* d = (const float*)blob;
-  c.Pk = d + oPk; c.Pt = d + oPt; c.Vt = d + oVt; c.Wt = d + oWt; c.Wv = d + oWv; c.Jt = d + oJt; c.Jsd = d + oJsd; c.pose_mean = d + oPm; c.Bhi = d + oBh; c.Blo = d + oBl; c.Ph = d + oPh; c.Pl = d + oPl;
+  c.Vt = d + oVt; c.Wt = d + oWt; c.Wv = d + oWv; c.Jt = d + oJt; c.Jsd = d + oJsd; c.pose_mean = d + oPm; c.Bhi = d + oBh; c.Blo = d + oBl; c.Ph = d + oPh; c.Pl = d + oPl;
   hb_mano* hm = new hb_mano;
   hm->c = c; hm->device = device; hm->blob = blob;
   *out = hm;

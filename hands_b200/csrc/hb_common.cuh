@@ -20,12 +20,10 @@ constexpr int AS = 192;            // 16 joints x (3x4) skinning transforms per 
 constexpr int VPB = 160;
 constexpr int NSLICE = 5;
 constexpr int VP = VPB * NSLICE;   // 800
-constexpr int HBF = 16;            // hands per CTA in the skinning kernels (feature tile layout depends on it)
+constexpr int HBF = 16;            // hands per skinning group (the A / OFF workspace regions are laid out by it)
 
 // MANO constants, device-resident, re-laid-out for coalesced access (built by hb_mano_create).
 struct ManoConst {
-  const float* Pk;    // [NP][3][VP]   Pk[p][k][v] = posedirs[p][3v+k] (p<135) | shapedirs[v][k][p-135]
-  const float* Pt;    // [3][VP][FS]   same values, p fastest (for the backward reduction over vertices)
   const float* Vt;    // [3][VP]       v_template transposed
   const float* Wt;    // [16][VP]      lbs_weights transposed
   const float* Wv;    // [VP][16]      lbs_weights, vertex-major, zero-padded
@@ -69,7 +67,6 @@ int launch_blend_tc(const float* Fhi, const float* Flo, const float* Bhi, const 
 constexpr int G_MAXSPLIT = 4;   // split-K parts of the backward feature contraction (partials [part][B128][160] in the workspace)
 int gfeat_nsplit(int B);
 int launch_gfeat_tc(const float* gvh, const float* gvl, const float* Ph, const float* Pl, int B, float* gF, cudaStream_t st);
-extern int g_mano_tc;   // 1: blendshape contraction on tcgen05 (mano_tc.cu); 0: register-tiled FFMA
 
 static inline bool aligned8(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 7u) == 0; }
 

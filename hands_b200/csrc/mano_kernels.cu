@@ -3,43 +3,44 @@
 // Two kernel families:
 //   * pose kernels  : one thread per (hand, joint), 16-lane shuffle groups walk the kinematic tree.
 //                     log map (rot.py:118-193) -> Rodrigues -> folded joint regression -> chain ->
-//                     skinning transforms A, blendshape feature row F, the 16 posed joints with
-//                     camera translation and 2D projection (mano_head.py:42-51).
+//                     skinning transforms A, the blendshape feature row as TF32 hi/lo slabs, the 16 posed joints
+//                     with camera translation and 2D projection (mano_head.py:42-51).
+//   * blendshapes   : v_posed = v_template + [posedirs; shapedirs^T]^T F on tcgen05, 3xTF32 (K3+K5, mano_tc.cu).
 //   * skin kernels  : one thread per vertex, HBF hands per CTA, 5 vertex slices.
-//                     v_posed = v_template + [posedirs; shapedirs^T]^T F   (K3+K5, register-tiled)
 //                     T_v = sum_j W[v,j] A_j ; x = T_v [v_posed;1]          (K7)
 //                     finger-tip joints + projection (K8, K11), coalesced stores through smem.
-//                     Backward recomputes v_posed and T_v and reduces dA, dF over vertices in smem.
-// Workspace layout (floats), G = ceil(B/HBF):
-//   F   [G][FS][HBF]      feature rows, hand fastest (skin kernels read it with LDS.128 broadcasts)
-//   A   [G][HBF][AS]      16 x (3x4) transforms
-//   OFF [G][HBF][8]       t1 (transl or 0), t2 (cam_t or 0), pad
-//   backward only: gF [NSLICE][G][HBF][FS], gA [NSLICE][G][HBF][AS], gO [NSLICE][G][HBF][8]
-#include <cstdlib>
+//                     Backward recomputes T_v, reduces dA over vertices in smem and writes dL/dv_posed as TF32 hi/lo
+//                     slabs; the feature gradient is their contraction with the basis on tcgen05 (mano_tc.cu).
+// Workspace layout (floats), G = ceil(B/HBF), G128 = ceil(B/128).  The forward's regions are a prefix of the backward's,
+// so a backward-sized workspace holds what the forward wrote where hb_mano_head_bwd_reuse() looks for it.
+//   A   [G][HBF][AS]          16 x (3x4) transforms
+//   OFF [G][HBF][8]           t1 (transl or 0), t2 (cam_t or 0), pad
+//   fh, fl [G128][19][1024]   feature rows, TF32 hi / lo parts in UMMA slab order
+//   vp  [G128*128][2400]      v_posed, coordinate-major per hand
+//   backward only:
+//   gA  [NSLICE][G][HBF][AS], gO [NSLICE][G][HBF][8]   per-slice partials
+//   gvh, gvl [G128][300][1024]                         dL/dv_posed, TF32 hi / lo parts in UMMA slab order
+//   gfeat [G_MAXSPLIT][G128*128][160]                  split-K partials of the feature gradient
 #include "hb_common.cuh"
 #include "pose_math.cuh"
 
 namespace hb {
 
 __host__ __device__ inline size_t ws_groups(int B) { return (size_t)(B + HBF - 1) / HBF; }
-__host__ __device__ inline size_t ws_F(int B) { (void)B; return 0; }
-__host__ __device__ inline size_t ws_A(int B) { return ws_groups(B) * FS * HBF; }
-__host__ __device__ inline size_t ws_OFF(int B) { return ws_A(B) + ws_groups(B) * HBF * AS; }
-__host__ __device__ inline size_t ws_fwd_end(int B) { return ws_OFF(B) + ws_groups(B) * HBF * 8; }
-__host__ __device__ inline size_t ws_gF(int B) { return ws_fwd_end(B); }
-__host__ __device__ inline size_t ws_gA(int B) { return ws_gF(B) + (size_t)NSLICE * ws_groups(B) * HBF * FS; }
-__host__ __device__ inline size_t ws_gO(int B) { return ws_gA(B) + (size_t)NSLICE * ws_groups(B) * HBF * AS; }
-__host__ __device__ inline size_t ws_bwd_end(int B) { return ws_gO(B) + (size_t)NSLICE * ws_groups(B) * HBF * 8; }
-// tensor-core path regions (after the FFMA regions): feature slabs hi/lo [G128][19][1024], v_posed [G128*128][2400]
 __host__ __device__ inline size_t ws_g128(int B) { return (size_t)(B + 127) / 128; }
-__host__ __device__ inline size_t ws_tc_base(int B, int backward) { return backward ? ws_bwd_end(B) : ws_fwd_end(B); }
-__host__ __device__ inline size_t ws_tc_F(int B) { return ws_g128(B) * 19 * 1024; }
-__host__ __device__ inline size_t ws_tc_vp(int B) { return ws_g128(B) * 128 * 2400; }
-// backward only: dL/dv_posed slabs hi/lo [G128][300][1024] and the reduced feature gradient [G128*128][160]
-__host__ __device__ inline size_t ws_tc_gv(int B) { return ws_g128(B) * 300 * 1024; }
-__host__ __device__ inline size_t ws_tc_end(int B, int backward) {
-  return ws_tc_base(B, backward) + 2 * ws_tc_F(B) + ws_tc_vp(B) + (backward ? 2 * ws_tc_gv(B) + (size_t)G_MAXSPLIT * ws_g128(B) * 128 * 160 : 0);
-}
+__host__ __device__ inline size_t ws_A(int B) { (void)B; return 0; }
+__host__ __device__ inline size_t ws_OFF(int B) { return ws_A(B) + ws_groups(B) * HBF * AS; }
+__host__ __device__ inline size_t ws_fh(int B) { return ws_OFF(B) + ws_groups(B) * HBF * 8; }
+__host__ __device__ inline size_t ws_fl(int B) { return ws_fh(B) + ws_g128(B) * 19 * 1024; }
+__host__ __device__ inline size_t ws_vp(int B) { return ws_fl(B) + ws_g128(B) * 19 * 1024; }
+__host__ __device__ inline size_t ws_fwd_end(int B) { return ws_vp(B) + ws_g128(B) * 128 * 2400; }
+__host__ __device__ inline size_t ws_gA(int B) { return ws_fwd_end(B); }
+__host__ __device__ inline size_t ws_gO(int B) { return ws_gA(B) + (size_t)NSLICE * ws_groups(B) * HBF * AS; }
+__host__ __device__ inline size_t ws_gvh(int B) { return ws_gO(B) + (size_t)NSLICE * ws_groups(B) * HBF * 8; }
+__host__ __device__ inline size_t ws_gvl(int B) { return ws_gvh(B) + ws_g128(B) * 300 * 1024; }
+__host__ __device__ inline size_t ws_gfeat(int B) { return ws_gvl(B) + ws_g128(B) * 300 * 1024; }
+__host__ __device__ inline size_t ws_gfeat_part(int B) { return ws_g128(B) * 128 * 160; }
+__host__ __device__ inline size_t ws_bwd_end(int B) { return ws_gfeat(B) + (size_t)G_MAXSPLIT * ws_gfeat_part(B); }
 
 // -------------------------------------------------------------------------------------------
 // per-(hand, joint) forward state
@@ -64,7 +65,7 @@ struct JointState {
 struct PoseArgs {
   const float* pose; int fmt; const float* pre_rot; const float* betas;   // fmt: 0 axis-angle, 1 rotmat, 2+L 6D layout L
   const float* cam; const float* K; const float* transl; int B; float img_res; float min_s;
-  float* fh; float* fl;   // tensor-core feature slabs (hi / lo TF32 parts) or NULL
+  float* fh; float* fl;   // feature slabs (hi / lo TF32 parts) in the workspace
 };
 
 __device__ __forceinline__ float shfl16(float v, int src) { return __shfl_sync(0xffffffffu, v, src, 16); }
@@ -160,10 +161,10 @@ __global__ void __launch_bounds__(128) mano_pose_fwd_kernel(ManoConst c, PoseArg
   pose_forward(c, a, b, i, s);
   if (!live) return;
   const size_t g = b / HBF, h = b % HBF;
-  float* F = ws + ws_F(a.B) + g * FS * HBF;
   float* A = ws + ws_A(a.B) + (g * HBF + h) * AS + i * 12;
-  if (a.fh) {
-    // UMMA slab order: [group128][k-step][k-half][row-group][row][4]  (mano_tc.cu)
+  {
+    // feature row F = [R_1 - I, ..., R_15 - I, betas, 0 pad] in UMMA slab order: [group128][k-step][k-half][row-group][row][4]
+    // (mano_tc.cu)
     const size_t gb = (size_t)(b / 128) * 19 * 1024;
     const int hl = b % 128;
     const int rowoff = (hl >> 3) * 32 + (hl & 7) * 4;
@@ -178,14 +179,7 @@ __global__ void __launch_bounds__(128) mano_pose_fwd_kernel(ManoConst c, PoseArg
       a.fh[o] = hi; a.fl[o] = lo;
     }
   }
-  if (i > 0) {
-#pragma unroll
-    for (int k = 0; k < 9; ++k) F[((i - 1) * 9 + k) * HBF + h] = s.R[k] - ((k % 4 == 0) ? 1.f : 0.f);
-  } else {
-#pragma unroll
-    for (int l = 0; l < NB; ++l) F[(NPF + l) * HBF + h] = __ldg(a.betas + (size_t)b * NB + l);
-#pragma unroll
-    for (int l = NP; l < FS; ++l) F[l * HBF + h] = 0.f;
+  if (i == 0) {
     float* off = ws + ws_OFF(a.B) + (g * HBF + h) * 8;
 #pragma unroll
     for (int k = 0; k < 3; ++k) { off[k] = s.t1[k]; off[3 + k] = s.camt[k]; }
@@ -230,29 +224,6 @@ __device__ __forceinline__ int tip_slot(const ManoConst& c, int v) {
   return t;
 }
 
-// v_posed for one vertex and HBF hands: acc[h][k] = Vt[k][v] + sum_p Pk[p][k][v] * F[p][h]
-__device__ __forceinline__ void blend_gemm(const ManoConst& c, const float* __restrict__ Fs, int v, float (&acc)[HBF][3]) {
-  const float v0 = __ldg(c.Vt + 0 * VP + v), v1 = __ldg(c.Vt + 1 * VP + v), v2 = __ldg(c.Vt + 2 * VP + v);
-#pragma unroll
-  for (int h = 0; h < HBF; ++h) { acc[h][0] = v0; acc[h][1] = v1; acc[h][2] = v2; }
-  const float* pk = c.Pk + v;
-#pragma unroll 5
-  for (int p = 0; p < NP; ++p) {
-    const float p0 = __ldg(pk + (size_t)(p * 3 + 0) * VP);
-    const float p1 = __ldg(pk + (size_t)(p * 3 + 1) * VP);
-    const float p2 = __ldg(pk + (size_t)(p * 3 + 2) * VP);
-    const float4* f4 = reinterpret_cast<const float4*>(Fs + p * HBF);
-#pragma unroll
-    for (int q = 0; q < HBF / 4; ++q) {
-      const float4 f = f4[q];
-      acc[q * 4 + 0][0] = fmaf(p0, f.x, acc[q * 4 + 0][0]); acc[q * 4 + 0][1] = fmaf(p1, f.x, acc[q * 4 + 0][1]); acc[q * 4 + 0][2] = fmaf(p2, f.x, acc[q * 4 + 0][2]);
-      acc[q * 4 + 1][0] = fmaf(p0, f.y, acc[q * 4 + 1][0]); acc[q * 4 + 1][1] = fmaf(p1, f.y, acc[q * 4 + 1][1]); acc[q * 4 + 1][2] = fmaf(p2, f.y, acc[q * 4 + 1][2]);
-      acc[q * 4 + 2][0] = fmaf(p0, f.z, acc[q * 4 + 2][0]); acc[q * 4 + 2][1] = fmaf(p1, f.z, acc[q * 4 + 2][1]); acc[q * 4 + 2][2] = fmaf(p2, f.z, acc[q * 4 + 2][2]);
-      acc[q * 4 + 3][0] = fmaf(p0, f.w, acc[q * 4 + 3][0]); acc[q * 4 + 3][1] = fmaf(p1, f.w, acc[q * 4 + 3][1]); acc[q * 4 + 3][2] = fmaf(p2, f.w, acc[q * 4 + 3][2]);
-    }
-  }
-}
-
 // T (3x4, row-major 12) = sum_j w[j] * A[j].  Packed f32x2 FMAs (sm_100 FFMA2: two IEEE fp32 FMAs per issue slot; each lane is
 // exactly fmaf(w[j], A[j][k], T[k]), so the result is bit-identical to the scalar form): 6 instead of 12 FMA issues per joint.
 __device__ __forceinline__ void blend_transforms(const float* __restrict__ Ah, const float (&w)[NJ], float (&T)[12]) {
@@ -274,12 +245,10 @@ __device__ __forceinline__ void blend_transforms(const float* __restrict__ Ah, c
 
 struct SkinFwdOut { float* vertices; float* v3d; float* joints3d; float* j3d_cam; float* j2d; };
 
-template <bool USE_VP>
-__global__ void __launch_bounds__(VPB, USE_VP ? 5 : 3) mano_skin_fwd_kernel(ManoConst c, const float* __restrict__ ws, const float* __restrict__ Kmat,
-                                                            int B, float img_res, SkinFwdOut o, const float* __restrict__ vp) {
+__global__ void __launch_bounds__(VPB, 5) mano_skin_fwd_kernel(ManoConst c, const float* __restrict__ ws, const float* __restrict__ Kmat,
+                                                                int B, float img_res, SkinFwdOut o, const float* __restrict__ vp) {
   extern __shared__ __align__(16) float smem[];
-  float* Fs = smem;                                // [FS][HBF]  (not needed in tensor-core mode)
-  float* As = Fs + (USE_VP ? 0 : FS * HBF);        // [HBF][AS]
+  float* As = smem;                                // [HBF][AS]
   float* Os = As + HBF * AS;                       // [HBF][8]
   float* Xs = Os + HBF * 8;                        // [HBF][XS]
   const int tid = threadIdx.x;
@@ -287,31 +256,20 @@ __global__ void __launch_bounds__(VPB, USE_VP ? 5 : 3) mano_skin_fwd_kernel(Mano
   const int v = slice * VPB + tid;
   const int b0 = g * HBF;
   {
-    const float4* srcF = reinterpret_cast<const float4*>(ws + ws_F(B) + (size_t)g * FS * HBF);
     const float4* srcA = reinterpret_cast<const float4*>(ws + ws_A(B) + (size_t)g * HBF * AS);
     const float4* srcO = reinterpret_cast<const float4*>(ws + ws_OFF(B) + (size_t)g * HBF * 8);
-    if (!USE_VP) for (int idx = tid; idx < FS * HBF / 4; idx += VPB) reinterpret_cast<float4*>(Fs)[idx] = srcF[idx];
     // (only the transforms of this CTA's share of the group's hands)
     const int a0 = (int)blockIdx.z * (HBF / (int)gridDim.z) * AS / 4, a1 = a0 + (HBF / (int)gridDim.z) * AS / 4;
     for (int idx = a0 + tid; idx < a1; idx += VPB) reinterpret_cast<float4*>(As)[idx] = srcA[idx];
     for (int idx = tid; idx < HBF * 8 / 4; idx += VPB) reinterpret_cast<float4*>(Os)[idx] = srcO[idx];
   }
   __syncthreads();
-  if (USE_VP) {
-    // v_posed comes from the tensor-core kernel: [hand][k][800] coordinate-major, coalesced over vertices
+  // v_posed comes from the tensor-core kernel: [hand][k][800] coordinate-major, coalesced over vertices
 #pragma unroll 4
-    for (int h = (int)blockIdx.z * (HBF / (int)gridDim.z); h < ((int)blockIdx.z + 1) * (HBF / (int)gridDim.z); ++h) {
-      const int b = min(b0 + h, B - 1);
-      const float* src = vp + (size_t)b * (3 * VP) + v;
-      Xs[h * XS + 3 * tid + 0] = __ldg(src); Xs[h * XS + 3 * tid + 1] = __ldg(src + VP); Xs[h * XS + 3 * tid + 2] = __ldg(src + 2 * VP);
-    }
-  } else {
-    float acc[HBF][3];
-    blend_gemm(c, Fs, v, acc);
-#pragma unroll
-    for (int h = 0; h < HBF; ++h) {
-      Xs[h * XS + 3 * tid + 0] = acc[h][0]; Xs[h * XS + 3 * tid + 1] = acc[h][1]; Xs[h * XS + 3 * tid + 2] = acc[h][2];
-    }
+  for (int h = (int)blockIdx.z * (HBF / (int)gridDim.z); h < ((int)blockIdx.z + 1) * (HBF / (int)gridDim.z); ++h) {
+    const int b = min(b0 + h, B - 1);
+    const float* src = vp + (size_t)b * (3 * VP) + v;
+    Xs[h * XS + 3 * tid + 0] = __ldg(src); Xs[h * XS + 3 * tid + 1] = __ldg(src + VP); Xs[h * XS + 3 * tid + 2] = __ldg(src + 2 * VP);
   }
   float w[NJ];
 #pragma unroll
@@ -371,22 +329,16 @@ __global__ void __launch_bounds__(VPB, USE_VP ? 5 : 3) mano_skin_fwd_kernel(Mano
 struct SkinBwdIn { const float* g_vertices; const float* g_v3d; const float* g_joints3d; const float* g_j3d_cam; const float* g_j2d; };
 
 constexpr int HSUB = 8;           // hands per reduction pass of the backward kernel
-constexpr int GPS = HSUB + 0;     // g_p tile row length (hand fastest)
 
-template <bool USE_VP>
-__global__ void __launch_bounds__(VPB, USE_VP ? 5 : 2) mano_skin_bwd_kernel(ManoConst c, float* __restrict__ ws, const float* __restrict__ Kmat,
-                                                            int B, float img_res, SkinBwdIn gi, const float* __restrict__ vp,
-                                                            float* __restrict__ gvh, float* __restrict__ gvl) {
+__global__ void __launch_bounds__(VPB, 5) mano_skin_bwd_kernel(ManoConst c, float* __restrict__ ws, const float* __restrict__ Kmat,
+                                                                int B, float img_res, SkinBwdIn gi, const float* __restrict__ vp,
+                                                                float* __restrict__ gvh, float* __restrict__ gvl) {
   extern __shared__ __align__(16) float smem[];
-  // (in tensor-core mode the feature tile Fs and the dL/dv_posed tile Gp are not needed: the contraction and its
-  //  transpose run in mano_tc.cu)
-  float* Fs = smem;                                    // [FS][HBF]
-  float* As = Fs + (USE_VP ? 0 : FS * HBF);            // [HBF][AS]
+  float* As = smem;                                    // [HBF][AS]
   float* Os = As + HBF * AS;                           // [HBF][8]
   float* Vs = Os + HBF * 8;                            // [HSUB][XS]   v_posed
   float* Gv = Vs + HSUB * XS;                          // [HSUB][XS]   dL/dvertex
-  float* Gp = Gv + HSUB * XS;                          // [VPB*3][HSUB] dL/dv_posed, hand fastest
-  float* Og = Gp + (USE_VP ? 0 : VPB * 3 * HSUB);      // [HSUB][8]    per-hand sums of g_vertices / g_v3d (+ tip joints)
+  float* Og = Gv + HSUB * XS;                          // [HSUB][8]    per-hand sums of g_vertices / g_v3d (+ tip joints)
   float* Ogw = Og + HSUB * 8;                          // [VPB/32][HSUB][8] the same per warp (summed in warp order: deterministic)
   const int tid = threadIdx.x;
   const int g = blockIdx.x, slice = blockIdx.y;
@@ -394,18 +346,14 @@ __global__ void __launch_bounds__(VPB, USE_VP ? 5 : 2) mano_skin_bwd_kernel(Mano
   const int b0 = g * HBF;
   const size_t G = ws_groups(B);
   {
-    const float4* srcF = reinterpret_cast<const float4*>(ws + ws_F(B) + (size_t)g * FS * HBF);
     const float4* srcA = reinterpret_cast<const float4*>(ws + ws_A(B) + (size_t)g * HBF * AS);
     const float4* srcO = reinterpret_cast<const float4*>(ws + ws_OFF(B) + (size_t)g * HBF * 8);
-    if (!USE_VP) for (int idx = tid; idx < FS * HBF / 4; idx += VPB) reinterpret_cast<float4*>(Fs)[idx] = srcF[idx];
     // (only the transforms of this CTA's share of the group's hands)
     const int a0 = gridDim.z > 1 ? (int)blockIdx.z * HSUB * AS / 4 : 0, a1 = gridDim.z > 1 ? a0 + HSUB * AS / 4 : HBF * AS / 4;
     for (int idx = a0 + tid; idx < a1; idx += VPB) reinterpret_cast<float4*>(As)[idx] = srcA[idx];
     for (int idx = tid; idx < HBF * 8 / 4; idx += VPB) reinterpret_cast<float4*>(Os)[idx] = srcO[idx];
   }
   __syncthreads();
-  float acc[USE_VP ? 1 : HBF][3];
-  if (!USE_VP) blend_gemm(c, Fs, v, reinterpret_cast<float (&)[HBF][3]>(acc));
   float w[NJ];
 #pragma unroll
   for (int j = 0; j < NJ; ++j) w[j] = __ldg(c.Wt + j * VP + v);
@@ -419,16 +367,10 @@ __global__ void __launch_bounds__(VPB, USE_VP ? 5 : 2) mano_skin_bwd_kernel(Mano
     if (gridDim.z > 1 && sub != (int)blockIdx.z) continue;
 #pragma unroll
     for (int hh = 0; hh < HSUB; ++hh) {
-      if (USE_VP) {
-        // v_posed from the tensor-core kernel: [hand][k][800], coalesced over vertices
-        const int b = min(b0 + sub * HSUB + hh, B - 1);
-        const float* src = vp + (size_t)b * (3 * VP) + v;
-        Vs[hh * XS + 3 * tid + 0] = __ldg(src); Vs[hh * XS + 3 * tid + 1] = __ldg(src + VP); Vs[hh * XS + 3 * tid + 2] = __ldg(src + 2 * VP);
-      } else {
-        Vs[hh * XS + 3 * tid + 0] = acc[USE_VP ? 0 : sub * HSUB + hh][0];
-        Vs[hh * XS + 3 * tid + 1] = acc[USE_VP ? 0 : sub * HSUB + hh][1];
-        Vs[hh * XS + 3 * tid + 2] = acc[USE_VP ? 0 : sub * HSUB + hh][2];
-      }
+      // v_posed from the tensor-core kernel: [hand][k][800], coalesced over vertices
+      const int b = min(b0 + sub * HSUB + hh, B - 1);
+      const float* src = vp + (size_t)b * (3 * VP) + v;
+      Vs[hh * XS + 3 * tid + 0] = __ldg(src); Vs[hh * XS + 3 * tid + 1] = __ldg(src + VP); Vs[hh * XS + 3 * tid + 2] = __ldg(src + 2 * VP);
     }
     __syncthreads();
     // ---- phase L: per vertex, per hand: T_v, upstream vertex gradient, g_p = R_v^T gV
@@ -485,7 +427,7 @@ __global__ void __launch_bounds__(VPB, USE_VP ? 5 : 2) mano_skin_bwd_kernel(Mano
         gp[2] = T[2] * gv[0] + T[6] * gv[1] + T[10] * gv[2];
       }
       Gv[hh * XS + 3 * tid + 0] = gv[0]; Gv[hh * XS + 3 * tid + 1] = gv[1]; Gv[hh * XS + 3 * tid + 2] = gv[2];
-      if (USE_VP) {
+      {
         // dL/dv_posed goes to the tensor-core reduction (mano_gfeat_tc_kernel) as TF32 hi/lo UMMA slabs:
         // [group128][k-step = c'/8][k-half][row-group][row][4], c' = k*800 + v
         const int hl = b % 128;
@@ -497,8 +439,6 @@ __global__ void __launch_bounds__(VPB, USE_VP ? 5 : 2) mano_skin_bwd_kernel(Mano
           const float hi = tf32_round(gp[k]);
           gvh[o] = hi; gvl[o] = tf32_round(gp[k] - hi);
         }
-      } else {
-        Gp[(3 * tid + 0) * GPS + hh] = gp[0]; Gp[(3 * tid + 1) * GPS + hh] = gp[1]; Gp[(3 * tid + 2) * GPS + hh] = gp[2];
       }
       // per-hand sums: warp shuffle tree, one slot per warp; the slots are added in warp order after the barrier (no float
       // atomics: g_cam / g_transl do not depend on the order the warps arrive in)
@@ -545,34 +485,6 @@ __global__ void __launch_bounds__(VPB, USE_VP ? 5 : 2) mano_skin_bwd_kernel(Mano
 #pragma unroll
       for (int k = 0; k < 12; ++k) dst[k] = ga[k];
     }
-    // ---- phase F: gF[h][p] = sum_{k,v} Pt[k][v][p] g_p[v][k][h]                    thread = p
-    if (!USE_VP && tid < FS) {
-      float gf[HSUB];
-#pragma unroll
-      for (int hh = 0; hh < HSUB; ++hh) gf[hh] = 0.f;
-      if (tid < NP) {
-#pragma unroll
-        for (int k = 0; k < 3; ++k) {
-          const float* pt = c.Pt + ((size_t)k * VP + slice * VPB) * FS + tid;
-#pragma unroll 4
-          for (int vv = 0; vv < VPB; ++vv) {
-            const float pv = __ldg(pt + (size_t)vv * FS);
-            const float4* g4 = reinterpret_cast<const float4*>(Gp + (3 * vv + k) * GPS);
-#pragma unroll
-            for (int q = 0; q < HSUB / 4; ++q) {
-              const float4 gq = g4[q];
-              gf[q * 4 + 0] = fmaf(pv, gq.x, gf[q * 4 + 0]); gf[q * 4 + 1] = fmaf(pv, gq.y, gf[q * 4 + 1]);
-              gf[q * 4 + 2] = fmaf(pv, gq.z, gf[q * 4 + 2]); gf[q * 4 + 3] = fmaf(pv, gq.w, gf[q * 4 + 3]);
-            }
-          }
-        }
-      }
-#pragma unroll
-      for (int hh = 0; hh < HSUB; ++hh) {
-        const int h = sub * HSUB + hh;
-        ws[ws_gF(B) + (((size_t)slice * G + g) * HBF + h) * FS + tid] = gf[hh];
-      }
-    }
     if (tid < HSUB * 8) {   // written by this same thread above
       const int hh = tid >> 3, k = tid & 7;
       const int h = sub * HSUB + hh;
@@ -613,32 +525,21 @@ __global__ void __launch_bounds__(128, 4) mano_pose_bwd_kernel(ManoConst c, Pose
     const float* pa = ws + ws_gA(a.B) + row * AS + i * 12;
 #pragma unroll
     for (int k = 0; k < 12; ++k) gA[k] += pa[k];
-    const float* pf = ws + ws_gF(a.B) + row * FS;
-    if (i > 0) {
-      if (!gFt) {
-#pragma unroll
-        for (int k = 0; k < 9; ++k) gFr[k] += pf[(i - 1) * 9 + k];
-      }
-    } else {
-      if (!gFt) {
-#pragma unroll
-        for (int l = 0; l < NB; ++l) gbeta[l] += pf[NPF + l];
-      }
+    if (i == 0) {
       const float* po = ws + ws_gO(a.B) + row * 8;
 #pragma unroll
       for (int k = 0; k < 6; ++k) gO[k] += po[k];
     }
   }
-  if (gFt) {   // feature gradient reduced over all vertices by the tensor-core kernel: split-K partials [part][hand][160], added in order
-    for (int part = 0; part < gf_parts; ++part) {
-      const float* pf = gFt + (size_t)part * gf_stride + (size_t)b * 160;
-      if (i > 0) {
+  // feature gradient reduced over all vertices by the tensor-core kernel: split-K partials [part][hand][160], added in order
+  for (int part = 0; part < gf_parts; ++part) {
+    const float* pf = gFt + (size_t)part * gf_stride + (size_t)b * 160;
+    if (i > 0) {
 #pragma unroll
-        for (int k = 0; k < 9; ++k) gFr[k] += __ldg(pf + (i - 1) * 9 + k);
-      } else {
+      for (int k = 0; k < 9; ++k) gFr[k] += __ldg(pf + (i - 1) * 9 + k);
+    } else {
 #pragma unroll
-        for (int l = 0; l < NB; ++l) gbeta[l] += __ldg(pf + NPF + l);
-      }
+      for (int l = 0; l < NB; ++l) gbeta[l] += __ldg(pf + NPF + l);
     }
   }
   // gradient arriving at this posed joint: joints3d = t + t1 ; j3d_cam = joints3d + cam_t ; j2d = proj(j3d_cam)
@@ -919,7 +820,7 @@ using namespace hb;
 
 extern "C" size_t hb_mano_workspace_bytes(int B, int backward) {
   if (B <= 0) return 0;
-  return sizeof(float) * ws_tc_end(B, backward);
+  return sizeof(float) * (backward ? ws_bwd_end(B) : ws_fwd_end(B));
 }
 
 static int check_common(const hb_mano* h, const float* pose, const float* betas, const float* cam, const float* K, int B,
@@ -931,23 +832,13 @@ static int check_common(const hb_mano* h, const float* pose, const float* betas,
   return 0;
 }
 
-static bool use_tc() {
-  if (g_mano_tc < 0) {
-    const char* e = getenv("HB_MANO_TC");
-    g_mano_tc = (e && e[0] == '0') ? 0 : 1;
-  }
-  return g_mano_tc == 1;
-}
-
 // CTAs per (16-hand group, vertex slice) of the skinning kernels: the group's hands are split over two CTAs (shorter serial
 // chain per CTA, twice the CTAs in flight).  Measured fwd+bwd of one side, 1 vs 2: 1024 hands 162 -> 145 us, 2048 221 -> 207,
 // 4096 344 -> 337, 8192 626 -> 614.
 constexpr unsigned kSkinHsplit = 2;
 
-static const size_t kSkinFwdSmem = sizeof(float) * (FS * HBF + HBF * AS + HBF * 8 + HBF * XS);
-static const size_t kSkinFwdSmemTc = sizeof(float) * (HBF * AS + HBF * 8 + HBF * XS);
-static const size_t kSkinBwdSmem = sizeof(float) * (FS * HBF + HBF * AS + HBF * 8 + 2 * HSUB * XS + VPB * 3 * HSUB + HSUB * 8 + (VPB / 32) * HSUB * 8);
-static const size_t kSkinBwdSmemTc = sizeof(float) * (HBF * AS + HBF * 8 + 2 * HSUB * XS + HSUB * 8 + (VPB / 32) * HSUB * 8);
+static const size_t kSkinFwdSmem = sizeof(float) * (HBF * AS + HBF * 8 + HBF * XS);
+static const size_t kSkinBwdSmem = sizeof(float) * (HBF * AS + HBF * 8 + 2 * HSUB * XS + HSUB * 8 + (VPB / 32) * HSUB * 8);
 
 extern "C" int hb_mano_head_fwd(const hb_mano* h, const float* pose, int pose_format, const float* pre_rot, const float* betas,
                                 const float* cam, const float* K, const float* transl, int B, float img_res, float min_s,
@@ -962,29 +853,20 @@ extern "C" int hb_mano_head_fwd(const hb_mano* h, const float* pose, int pose_fo
   if ((vertices && !aligned8(vertices)) || (v3d_cam && !aligned8(v3d_cam))) { set_error("hb_mano_head_fwd: vertex outputs must be 8-byte aligned"); return HB_E_ALIGN; }
   cudaStream_t st = (cudaStream_t)stream;
   float* ws = (float*)workspace;
-  const bool tc = use_tc();
-  // a backward-sized workspace is laid out as the backward expects it, so hb_mano_head_bwd_reuse() can pick the forward's
-  // feature rows, skinning transforms and v_posed up instead of recomputing them
-  const int lay = workspace_bytes >= hb_mano_workspace_bytes(B, 1) ? 1 : 0;
-  float* fh = tc ? ws + ws_tc_base(B, lay) : nullptr;
-  float* fl = tc ? fh + ws_tc_F(B) : nullptr;
-  float* vpo = tc ? fl + ws_tc_F(B) : nullptr;
+  float* fh = ws + ws_fh(B);
+  float* fl = ws + ws_fl(B);
+  float* vpo = ws + ws_vp(B);
   PoseArgs a{pose, pose_format, pre_rot, betas, cam, K, transl, B, img_res, min_s, fh, fl};
   mano_pose_fwd_kernel<<<(B + 7) / 8, 128, 0, st>>>(h->c, a, ws, joints3d, j3d_cam, j2d_norm, cam_t);
   g_launches++;
   rc = check_launch("mano_pose_fwd_kernel");
   if (rc) return rc;
+  rc = launch_blend_tc(fh, fl, h->c.Bhi, h->c.Blo, h->c.Vt, B, vpo, st);
+  if (rc) return rc;
   SkinFwdOut o{vertices, v3d_cam, joints3d, j3d_cam, j2d_norm};
   dim3 grid((unsigned)ws_groups(B), NSLICE, kSkinHsplit);
-  if (tc) {
-    rc = launch_blend_tc(fh, fl, h->c.Bhi, h->c.Blo, h->c.Vt, B, vpo, st);
-    if (rc) return rc;
-    HB_CUDA(cudaFuncSetAttribute(mano_skin_fwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSkinFwdSmemTc));
-    mano_skin_fwd_kernel<true><<<grid, VPB, kSkinFwdSmemTc, st>>>(h->c, ws, K, B, img_res, o, vpo);
-  } else {
-    HB_CUDA(cudaFuncSetAttribute(mano_skin_fwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSkinFwdSmem));
-    mano_skin_fwd_kernel<false><<<grid, VPB, kSkinFwdSmem, st>>>(h->c, ws, K, B, img_res, o, nullptr);
-  }
+  HB_CUDA(cudaFuncSetAttribute(mano_skin_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSkinFwdSmem));
+  mano_skin_fwd_kernel<<<grid, VPB, kSkinFwdSmem, st>>>(h->c, ws, K, B, img_res, o, vpo);
   g_launches++;
   return check_launch("mano_skin_fwd_kernel");
 }
@@ -1003,42 +885,32 @@ static int mano_head_bwd_impl(const hb_mano* h, const float* pose, int pose_form
   if (pre_rot && !pose_format) { set_error("hb_mano_head_bwd: pre_rot needs rotation-matrix or 6D pose input"); return HB_E_ARG; }
   cudaStream_t st = (cudaStream_t)stream;
   float* ws = (float*)workspace;
-  const bool tc = use_tc();
-  float* fh = tc ? ws + ws_tc_base(B, 1) : nullptr;
-  float* fl = tc ? fh + ws_tc_F(B) : nullptr;
-  float* vpo = tc ? fl + ws_tc_F(B) : nullptr;
-  float* gvh = tc ? vpo + ws_tc_vp(B) : nullptr;
-  float* gvl = tc ? gvh + ws_tc_gv(B) : nullptr;
-  float* gft = tc ? gvl + ws_tc_gv(B) : nullptr;
+  float* fh = ws + ws_fh(B);
+  float* fl = ws + ws_fl(B);
+  float* vpo = ws + ws_vp(B);
+  float* gvh = ws + ws_gvh(B);
+  float* gvl = ws + ws_gvl(B);
+  float* gft = ws + ws_gfeat(B);
   PoseArgs a{pose, pose_format, pre_rot, betas, cam, K, transl, B, img_res, min_s, fh, fl};
   if (!reuse) {
     mano_pose_fwd_kernel<<<(B + 7) / 8, 128, 0, st>>>(h->c, a, ws, nullptr, nullptr, nullptr, nullptr);
     g_launches++;
     rc = check_launch("mano_pose_fwd_kernel");
     if (rc) return rc;
+    rc = launch_blend_tc(fh, fl, h->c.Bhi, h->c.Blo, h->c.Vt, B, vpo, st);
+    if (rc) return rc;
   }
   SkinBwdIn gi{g_vertices, g_v3d_cam, g_joints3d, g_j3d_cam, g_j2d_norm};
   dim3 grid((unsigned)ws_groups(B), NSLICE, kSkinHsplit);
-  if (tc) {
-    if (!reuse) {
-      rc = launch_blend_tc(fh, fl, h->c.Bhi, h->c.Blo, h->c.Vt, B, vpo, st);
-      if (rc) return rc;
-    }
-    HB_CUDA(cudaFuncSetAttribute(mano_skin_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSkinBwdSmemTc));
-    mano_skin_bwd_kernel<true><<<grid, VPB, kSkinBwdSmemTc, st>>>(h->c, ws, K, B, img_res, gi, vpo, gvh, gvl);
-  } else {
-    HB_CUDA(cudaFuncSetAttribute(mano_skin_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSkinBwdSmem));
-    mano_skin_bwd_kernel<false><<<grid, VPB, kSkinBwdSmem, st>>>(h->c, ws, K, B, img_res, gi, nullptr, nullptr, nullptr);
-  }
+  HB_CUDA(cudaFuncSetAttribute(mano_skin_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSkinBwdSmem));
+  mano_skin_bwd_kernel<<<grid, VPB, kSkinBwdSmem, st>>>(h->c, ws, K, B, img_res, gi, vpo, gvh, gvl);
   g_launches++;
   rc = check_launch("mano_skin_bwd_kernel");
   if (rc) return rc;
-  if (tc) {
-    rc = launch_gfeat_tc(gvh, gvl, h->c.Ph, h->c.Pl, B, gft, st);
-    if (rc) return rc;
-  }
+  rc = launch_gfeat_tc(gvh, gvl, h->c.Ph, h->c.Pl, B, gft, st);
+  if (rc) return rc;
   PoseBwdArgs o{g_joints3d, g_j3d_cam, g_j2d_norm, g_cam_t, g_pose, g_betas, g_cam, g_transl, g_pre_rot};
-  mano_pose_bwd_kernel<<<(B + 7) / 8, 128, 0, st>>>(h->c, a, ws, o, gft, tc ? gfeat_nsplit(B) : 0, (size_t)ws_g128(B) * 128 * 160);
+  mano_pose_bwd_kernel<<<(B + 7) / 8, 128, 0, st>>>(h->c, a, ws, o, gft, gfeat_nsplit(B), ws_gfeat_part(B));
   g_launches++;
   return check_launch("mano_pose_bwd_kernel");
 }

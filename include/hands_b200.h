@@ -53,7 +53,7 @@ typedef struct hb_mano hb_mano; /* opaque: MANO constants of one hand side on on
 #define HB_ROT6D_COLS 1        /* src/models/hamer_light/geometry.py:47-62, src/models/handoccnet_light/mano_head.py:132-141: a1=x[0:3], a2=x[3:6], COLUMNS */
 #define HB_ROT6D_COLS_PAIRED 2 /* common/rot.py:367-381: a1=x[0,2,4], a2=x[1,3,5], COLUMNS */
 
-#define HB_VERSION 203 /* hb_version() of a matching binary */
+#define HB_VERSION 204 /* hb_version() of a matching binary */
 const char* hb_last_error_string(void);
 int hb_version(void);
 
@@ -68,10 +68,6 @@ int hb_mano_create(const float* v_template_host, const float* shapedirs_host, co
                    const float* J_regressor_host, const float* lbs_weights_host, const int32_t* parents_host,
                    const float* pose_mean_host, const int32_t* tip_ids_host, int device, hb_mano** out);
 int hb_mano_destroy(hb_mano* h);
-
-/* Blendshape contraction engine: 1 = tcgen05/TMEM tensor cores with 3xTF32 error compensation (default),
- * 0 = register-tiled FFMA.  Environment HB_MANO_TC=0/1 sets the initial value.  Returns the previous setting. */
-int hb_mano_set_tensor_core(int on);
 
 /* Bytes of scratch the fwd / bwd calls need for a batch of B hands. */
 size_t hb_mano_workspace_bytes(int B, int backward);
@@ -90,8 +86,8 @@ size_t hb_mano_workspace_bytes(int B, int backward);
  *   betas (B,10)   cam (B,3)=[s,tx,ty] or NULL   K (B,3,3) or NULL   transl (B,3) or NULL
  * Outputs (each or NULL): vertices (B,778,3), v3d_cam (B,778,3), joints3d (B,21,3),
  *   j3d_cam (B,21,3), j2d_norm (B,21,2), cam_t (B,3).  Camera outputs need cam and K.
- * Workspace: >= hb_mano_workspace_bytes(B, 0).  Given >= hb_mano_workspace_bytes(B, 1) bytes the forward lays its
- *   intermediates out as the backward expects them, which is what hb_mano_head_bwd_reuse() relies on. */
+ * Workspace: >= hb_mano_workspace_bytes(B, 0).  The forward's intermediates fill the start of the workspace in the
+ *   layout the backward reads, so a backward-sized workspace can be handed on to hb_mano_head_bwd_reuse(). */
 int hb_mano_head_fwd(const hb_mano* h, const float* pose, int pose_format, const float* pre_rot,
                      const float* betas, const float* cam, const float* K, const float* transl, int B,
                      float img_res, float min_s, float* vertices, float* v3d_cam, float* joints3d,
@@ -110,9 +106,9 @@ int hb_mano_head_bwd(const hb_mano* h, const float* pose, int pose_format, const
                      float* g_pre_rot, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Same backward when `workspace` is the very buffer a preceding hb_mano_head_fwd call on the SAME inputs was given, with
- * workspace_bytes >= hb_mano_workspace_bytes(B, 1) in both calls and nothing written to it in between: the forward's
- * feature rows, skinning transforms and v_posed (10.7 KB/hand) are picked up instead of recomputed (two launches and the
- * blendshape contraction less).  Results are bit-identical to hb_mano_head_bwd. */
+ * nothing written to it in between.  Like any backward it needs workspace_bytes >= hb_mano_workspace_bytes(B, 1).  The
+ * forward's skinning transforms, feature slabs and v_posed (11.6 KB/hand) are picked up instead of recomputed (two launches
+ * and the blendshape contraction less).  Results are bit-identical to hb_mano_head_bwd. */
 int hb_mano_head_bwd_reuse(const hb_mano* h, const float* pose, int pose_format, const float* pre_rot,
                            const float* betas, const float* cam, const float* K, const float* transl, int B,
                            float img_res, float min_s, const float* g_vertices, const float* g_v3d_cam,

@@ -34,6 +34,10 @@ def test_workspace_sizes_and_argument_errors():
     lib = _lib.load()
     assert lib.hb_mano_workspace_bytes(0, 0) == 0
     assert lib.hb_mano_workspace_bytes(1024, 1) > lib.hb_mano_workspace_bytes(1024, 0) > 0
+    # per hand, in floats: forward A 192 + OFF 8 + feature slabs 2 x 152 + v_posed 2400 = 2904; the backward adds the
+    # per-slice partials 5 x (192 + 8), the dL/dv_posed slabs 2 x 2400 and the split-K feature partials 4 x 160 = 6440
+    assert lib.hb_mano_workspace_bytes(1024, 0) == 1024 * 11616
+    assert lib.hb_mano_workspace_bytes(1024, 1) == 1024 * 37376
     assert lib.hb_pcl_bwd_workspace_bytes(8, 2, 3, 224) == 8 * 4 * 224 * 224 * 4  # one float4 gradient per intermediate pixel
     assert lib.hb_pcl_bwd_workspace_bytes(2 * 8192, 2, 3, 224) == 2 * 4096 * 4 * 224 * 224 * 4  # capped at 4096 images per chunk
     # argument validation happens before any CUDA call, so it is testable without a GPU
