@@ -52,6 +52,7 @@ SYMBOLS = {
     "hb_vec_loss_bwd": (ctypes.c_int, [ctypes.c_void_p] * 8 + [ctypes.c_int, ctypes.c_int] + [ctypes.c_void_p] * 5),
     "hb_axis_angle_to_matrix": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p]),
     "hb_mrrpe": (ctypes.c_int, [ctypes.c_void_p] * 5 + [ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
+    "hb_procrustes_metrics": (ctypes.c_int, [ctypes.c_void_p] * 2 + [ctypes.c_int, ctypes.c_int] + [ctypes.c_void_p] * 8),
     "hb_gt_process": (ctypes.c_int, [ctypes.c_void_p] * 4 + [ctypes.c_int, ctypes.c_float] + [ctypes.c_void_p] * 4),
     "hb_kpe_features": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int] + [ctypes.c_void_p] * 5),
     "hb_pcl_setup": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),

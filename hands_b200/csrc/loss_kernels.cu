@@ -132,6 +132,164 @@ __global__ void mrrpe_kernel(const float* __restrict__ pr, const float* __restri
   for (int k = 2; k < KS; ++k) p[k] = 0.f;
 }
 
+// Procrustes-aligned and root-relative point errors per hand (the HMR / ARCTIC compute_similarity_transform metric,
+// src/utils/eval_modules.py:136-219, which runs a numpy SVD per sample on the host; the contract is restated in
+// include/hands_b200.h and tests/procrustes_oracle.py::procrustes_errors).  One warp per hand, lane = point (strided):
+//   pass 1: moments of a_i = p_i - p_0, b_i = q_i - q_0 in fp64 (shifted by point 0, so camera-space offsets of metres
+//           cancel exactly in fp32 before anything is accumulated), folded into the centred C and var;
+//   solve : Horn's symmetric 4x4 matrix of C, cyclic Jacobi with a fixed sweep count in fp64 -> the unit quaternion of
+//           the proper rotation maximising trace(R C) (= V Z U^T of the SVD form, determinant correction included),
+//           computed redundantly by every lane (no broadcast, no divergence);
+//   pass 2: the row again (L1/L2), residuals s R X_i - Y_i in centred fp32 coordinates, `aligned`, the per-hand means.
+// Every reduction is a fixed butterfly: per-hand results do not depend on the batch they are computed in.
+constexpr int PA_SWEEPS = 6;   // quadratic convergence: the 4x4 off-diagonal is at rounding level after 4-5 sweeps
+
+__device__ __forceinline__ double warp_sum_d(double v) {
+#pragma unroll
+  for (int m = 16; m > 0; m >>= 1) v += __shfl_xor_sync(0xffffffffu, v, m);
+  return v;
+}
+
+struct ProcArgs {
+  const float* pred; const float* gt; const float* root_pred; const float* root_gt; const float* hv;
+  int B; int N; float* per_hand; float* aligned;
+};
+
+__global__ void __launch_bounds__(128) procrustes_kernel(ProcArgs a, float* __restrict__ partial) {
+  const int b = blockIdx.x * 4 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (b >= a.B) return;
+  const int N = a.N;
+  const float* P = a.pred + (size_t)b * N * 3;
+  const float* Q = a.gt + (size_t)b * N * 3;
+  const float p0[3] = {__ldg(P), __ldg(P + 1), __ldg(P + 2)}, q0[3] = {__ldg(Q), __ldg(Q + 1), __ldg(Q + 2)};
+
+  // pass 1: sum a, sum b, sum a b^T, sum |a|^2
+  double sa[3] = {0, 0, 0}, sb[3] = {0, 0, 0}, sab[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0}, saa = 0;
+  for (int i = lane; i < N; i += 32) {
+    double x[3], y[3];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) { x[k] = (double)(__ldg(P + 3 * i + k) - p0[k]); y[k] = (double)(__ldg(Q + 3 * i + k) - q0[k]); }
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+      sa[k] += x[k]; sb[k] += y[k]; saa = fma(x[k], x[k], saa);
+#pragma unroll
+      for (int l = 0; l < 3; ++l) sab[3 * k + l] = fma(x[k], y[l], sab[3 * k + l]);
+    }
+  }
+#pragma unroll
+  for (int k = 0; k < 3; ++k) { sa[k] = warp_sum_d(sa[k]); sb[k] = warp_sum_d(sb[k]); }
+#pragma unroll
+  for (int k = 0; k < 9; ++k) sab[k] = warp_sum_d(sab[k]);
+  saa = warp_sum_d(saa);
+  const double inv_n = 1.0 / (double)N;
+  double ma[3], mb[3], C[9];
+#pragma unroll
+  for (int k = 0; k < 3; ++k) { ma[k] = sa[k] * inv_n; mb[k] = sb[k] * inv_n; }
+#pragma unroll
+  for (int k = 0; k < 3; ++k)
+#pragma unroll
+    for (int l = 0; l < 3; ++l) C[3 * k + l] = sab[3 * k + l] - sa[k] * mb[l];   // sum X_k Y_l
+  const double var = saa - (sa[0] * ma[0] + sa[1] * ma[1] + sa[2] * ma[2]);       // sum |X|^2
+  const bool degenerate = !(var > 0.0);
+
+  // solve: Horn's matrix, Jacobi eigen-decomposition, quaternion of the largest eigenvalue
+  float sR[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+  if (!degenerate) {
+    const double Sxx = C[0], Sxy = C[1], Sxz = C[2], Syx = C[3], Syy = C[4], Syz = C[5], Szx = C[6], Szy = C[7], Szz = C[8];
+    double A[4][4] = {{Sxx + Syy + Szz, Syz - Szy, Szx - Sxz, Sxy - Syx},
+                      {Syz - Szy, Sxx - Syy - Szz, Sxy + Syx, Szx + Sxz},
+                      {Szx - Sxz, Sxy + Syx, -Sxx + Syy - Szz, Syz + Szy},
+                      {Sxy - Syx, Szx + Sxz, Syz + Szy, -Sxx - Syy + Szz}};
+    double V[4][4] = {{1, 0, 0, 0}, {0, 1, 0, 0}, {0, 0, 1, 0}, {0, 0, 0, 1}};
+    for (int sweep = 0; sweep < PA_SWEEPS; ++sweep) {
+#pragma unroll
+      for (int pq = 0; pq < 6; ++pq) {
+        const int p = pq < 3 ? 0 : (pq < 5 ? 1 : 2), q = pq < 3 ? pq + 1 : (pq < 5 ? pq - 1 : 3);
+        const double apq = A[p][q];
+        if (apq == 0.0) continue;
+        const double th = (A[q][q] - A[p][p]) / (2.0 * apq);
+        const double at = fabs(th);     // th^2 would overflow beyond 1e154; there t = 1/(2 th) to working precision
+        const double t = (th >= 0.0 ? 1.0 : -1.0) * (at > 1e150 ? 0.5 / at : 1.0 / (at + sqrt(fma(th, th, 1.0))));
+        const double c = rsqrt(fma(t, t, 1.0)), s = t * c;   // |t| <= 1
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {   // A <- A J (columns p, q)
+          const double akp = A[k][p], akq = A[k][q];
+          A[k][p] = c * akp - s * akq; A[k][q] = s * akp + c * akq;
+        }
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {   // A <- J^T A (rows p, q)
+          const double apk = A[p][k], aqk = A[q][k];
+          A[p][k] = c * apk - s * aqk; A[q][k] = s * apk + c * aqk;
+        }
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+          const double vkp = V[k][p], vkq = V[k][q];
+          V[k][p] = c * vkp - s * vkq; V[k][q] = s * vkp + c * vkq;
+        }
+      }
+    }
+    double qv[4] = {V[0][0], V[1][0], V[2][0], V[3][0]}, lmax = A[0][0];   // eigenvector of the largest eigenvalue
+#pragma unroll
+    for (int m = 1; m < 4; ++m)
+      if (A[m][m] > lmax) {
+        lmax = A[m][m];
+#pragma unroll
+        for (int k = 0; k < 4; ++k) qv[k] = V[k][m];
+      }
+    const double qn = 1.0 / sqrt(qv[0] * qv[0] + qv[1] * qv[1] + qv[2] * qv[2] + qv[3] * qv[3]);
+    const double w = qv[0] * qn, x = qv[1] * qn, y = qv[2] * qn, z = qv[3] * qn;
+    const double R[9] = {w * w + x * x - y * y - z * z, 2 * (x * y - w * z), 2 * (x * z + w * y),
+                         2 * (x * y + w * z), w * w - x * x + y * y - z * z, 2 * (y * z - w * x),
+                         2 * (x * z - w * y), 2 * (y * z + w * x), w * w - x * x - y * y + z * z};
+    const double sc = lmax / var;   // the largest eigenvalue of Horn's matrix is trace(R C) at the optimum
+#pragma unroll
+    for (int k = 0; k < 9; ++k) sR[k] = (float)(sc * R[k]);
+  }
+
+  // pass 2: residuals in centred coordinates (p^_i - q_i = s R X_i - Y_i), root-relative errors, aligned points
+  const float mpf[3] = {(float)ma[0], (float)ma[1], (float)ma[2]}, mqf[3] = {(float)mb[0], (float)mb[1], (float)mb[2]};
+  float rp[3], rq[3];
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    rp[k] = a.root_pred ? __ldg(a.root_pred + (size_t)b * 3 + k) : p0[k];
+    rq[k] = a.root_gt ? __ldg(a.root_gt + (size_t)b * 3 + k) : q0[k];
+  }
+  float* al = a.aligned ? a.aligned + (size_t)b * N * 3 : nullptr;
+  double pa_acc = 0.0, ra_acc = 0.0;
+  for (int i = lane; i < N; i += 32) {
+    float p[3], q[3], X[3], Y[3];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+      p[k] = __ldg(P + 3 * i + k); q[k] = __ldg(Q + 3 * i + k);
+      X[k] = (p[k] - p0[k]) - mpf[k]; Y[k] = (q[k] - q0[k]) - mqf[k];
+    }
+    float d2 = 0.f, e2 = 0.f;
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+      const float u = fmaf(sR[3 * k], X[0], fmaf(sR[3 * k + 1], X[1], sR[3 * k + 2] * X[2]));
+      const float d = u - Y[k], e = (p[k] - rp[k]) - (q[k] - rq[k]);
+      d2 = fmaf(d, d, d2); e2 = fmaf(e, e, e2);
+      if (al) al[3 * i + k] = degenerate ? __int_as_float(0x7fc00000) : (u + mqf[k]) + q0[k];
+    }
+    pa_acc += (double)sqrtf(d2);
+    ra_acc += (double)sqrtf(e2);
+  }
+  pa_acc = warp_sum_d(pa_acc);
+  ra_acc = warp_sum_d(ra_acc);
+  if (lane == 0) {
+    const bool valid = a.hv ? __ldg(a.hv + b) != 0.0f : true;
+    const float pa = (float)(pa_acc * inv_n), ra = (float)(ra_acc * inv_n), nan = __int_as_float(0x7fc00000);
+    if (a.per_hand) {
+      a.per_hand[(size_t)b * 2 + 0] = (valid && !degenerate) ? pa : nan;
+      a.per_hand[(size_t)b * 2 + 1] = valid ? ra : nan;
+    }
+    float* o = partial + (size_t)b * KS;
+    const bool use_pa = valid && !degenerate;
+    o[0] = use_pa ? pa : 0.f; o[1] = use_pa ? 1.f : 0.f; o[2] = valid ? ra : 0.f; o[3] = valid ? 1.f : 0.f;
+    o[4] = (valid && degenerate) ? 1.f : 0.f; o[5] = 0.f; o[6] = 0.f; o[7] = 0.f;
+  }
+}
+
 // GT-side glue of process_data_light (src/callbacks/process/process_arctic.py:42-65), one hand side:
 //   Tr0 = mean_j (j3d_full - joints_cano);  v3d_cam = vertices_cano + Tr0;  cam_t = j3d_full[:,0] - joints_cano[:,0];
 //   cam_t_wp = perspective_to_weak_perspective_torch(cam_t, (K00+K11)/2, img_res)   (common/camera.py:10-29)
@@ -382,6 +540,22 @@ extern "C" int hb_mrrpe(const float* j3d_cam_r, const float* j3d_cam_l, const fl
     mrrpe_kernel<<<(B + 127) / 128, 128, 0, st>>>(j3d_cam_r, j3d_cam_l, gt_j3d_cam_r, gt_j3d_cam_l, valid, B, partial);
     g_launches++;
     int rc = check_launch("mrrpe_kernel");
+    if (rc) return rc;
+  }
+  kp_reduce_kernel<<<1, 1024, 0, st>>>(partial, B, sums);
+  g_launches++;
+  return check_launch("kp_reduce_kernel");
+}
+
+extern "C" int hb_procrustes_metrics(const float* pred, const float* gt, int B, int N, const float* root_pred, const float* root_gt,
+                                     const float* hand_valid, float* per_hand, float* aligned, float* partial, float* sums, void* stream) {
+  if (B < 0 || !sums || (B > 0 && (!pred || !gt || !partial || N < 1))) { set_error("hb_procrustes_metrics: bad argument"); return HB_E_ARG; }
+  cudaStream_t st = (cudaStream_t)stream;
+  if (B > 0) {
+    ProcArgs a{pred, gt, root_pred, root_gt, hand_valid, B, N, per_hand, aligned};
+    procrustes_kernel<<<(B + 3) / 4, 128, 0, st>>>(a, partial);
+    g_launches++;
+    int rc = check_launch("procrustes_kernel");
     if (rc) return rc;
   }
   kp_reduce_kernel<<<1, 1024, 0, st>>>(partial, B, sums);

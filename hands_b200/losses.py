@@ -77,6 +77,44 @@ def mrrpe_sums(j3d_cam_r, j3d_cam_l, gt_j3d_cam_r, gt_j3d_cam_l, valid=None):
     return sums
 
 
+def procrustes_metrics(pred, gt, hand_valid=None, root_pred=None, root_gt=None, return_aligned=False):
+    """Procrustes-aligned and root-relative point errors of one hand side, as device partial sums (hb_procrustes_metrics):
+    the similarity fit of the HMR / ARCTIC `compute_similarity_transform` (src/utils/eval_modules.py:136-219, a numpy SVD
+    per sample there) solved per hand on the GPU, then the mean point distance after alignment (PA) and after subtracting
+    the root points (RA).  pred, gt (B,N,3) fp32 CUDA; root_pred, root_gt (B,3) or None (= point 0); hand_valid (B,) or
+    None.  On joints (N = 21) PA is PA-MPJPE and RA is MPJPE-RA; on `v3d.cam` vertices pass joint 0 of `j3d.cam` as the
+    roots and RA is the root-relative MPVPE.  A metric: inputs are detached, there is no gradient.
+
+    Returns (sums, per_hand[, aligned]): sums (8,) = [PA sum over valid non-degenerate hands, their count, RA sum over valid
+    hands, their count, valid hands left out as degenerate (var == 0, e.g. N = 1), 0, 0, 0]; per_hand (B,2) = [PA, RA],
+    NaN for invalid hands and PA NaN for degenerate ones; aligned (B,N,3) = s R pred + t.  With
+    `hands_b200.distributed.PackedMetrics`:
+
+        sums, _ = procrustes_metrics(pred["mano.j3d.cam.r"], gt["mano.j3d.cam.r"], gt["right_valid"])
+        pm.add("pa_mpjpe/r", sums[0], sums[1])
+        pm.add("mpjpe_ra/r", sums[2], sums[3])
+    """
+    lib = _lib.load()
+    d = lambda t: t.detach() if isinstance(t, torch.Tensor) else t  # noqa: E731
+    pred = _f32c(d(pred), "pred", (None, None, 3))
+    B, N = pred.shape[:2]
+    if N < 1:
+        raise ValueError("pred: expected at least one point per hand (N >= 1)")
+    gt = _f32c(d(gt), "gt", (B, N, 3))
+    root_pred, root_gt = _f32c(d(root_pred), "root_pred", (B, 3)), _f32c(d(root_gt), "root_gt", (B, 3))
+    hand_valid = _f32c(d(hand_valid), "hand_valid", (B,))
+    dev = pred.device
+    partial = torch.empty(max(B, 1), _lib.KP_SUMS, dtype=torch.float32, device=dev)
+    sums = torch.empty(_lib.KP_SUMS, dtype=torch.float32, device=dev)
+    per_hand = torch.empty(B, 2, dtype=torch.float32, device=dev)
+    aligned = torch.empty(B, N, 3, dtype=torch.float32, device=dev) if return_aligned else None
+    with torch.cuda.device(dev):
+        rc = lib.hb_procrustes_metrics(_ptr(pred), _ptr(gt), B, N, _ptr(root_pred), _ptr(root_gt), _ptr(hand_valid), _ptr(per_hand),
+                                       _ptr(aligned), _ptr(partial), _ptr(sums), _stream())
+    _lib.check(rc, "hb_procrustes_metrics")
+    return (sums, per_hand, aligned) if return_aligned else (sums, per_hand)
+
+
 class VectorLossFunction(torch.autograd.Function):
     """loss = mean_b,e [ valid*valid2*gate * ( ((pred - pred_minus) - (gt - gt_minus))^2 + (pred2 - (gt - gt_minus))^2 ) ].
     Gradients flow to pred, pred_minus and pred2; targets and masks are data.  (hb_vec_loss_fwd/bwd)"""

@@ -53,7 +53,7 @@ typedef struct hb_mano hb_mano; /* opaque: MANO constants of one hand side on on
 #define HB_ROT6D_COLS 1        /* src/models/hamer_light/geometry.py:47-62, src/models/handoccnet_light/mano_head.py:132-141: a1=x[0:3], a2=x[3:6], COLUMNS */
 #define HB_ROT6D_COLS_PAIRED 2 /* common/rot.py:367-381: a1=x[0,2,4], a2=x[1,3,5], COLUMNS */
 
-#define HB_VERSION 204 /* hb_version() of a matching binary */
+#define HB_VERSION 205 /* hb_version() of a matching binary */
 const char* hb_last_error_string(void);
 int hb_version(void);
 
@@ -184,6 +184,22 @@ int hb_axis_angle_to_matrix(const float* aa, int N, float* R, void* stream);
  * roots are joint 0 of the (B,21,3) arrays; valid (B) or NULL. */
 int hb_mrrpe(const float* j3d_cam_r, const float* j3d_cam_l, const float* gt_j3d_cam_r, const float* gt_j3d_cam_l,
              const float* valid, int B, float* partial, float* sums, void* stream);
+/* Procrustes-aligned and root-relative point errors (PA-MPJPE / PA-MPVPE, MPJPE-RA / root-relative MPVPE): the similarity
+ * fit of the HMR / ARCTIC compute_similarity_transform (src/utils/eval_modules.py:136-219, numpy SVD per sample there).
+ * For hand b with p_i = pred[b,i], q_i = gt[b,i], i < N:
+ *   mu_p, mu_q = means;  X_i = p_i - mu_p;  Y_i = q_i - mu_q;  var = sum |X_i|^2;  C = sum X_i Y_i^T
+ *   U, S, V^T = svd(C);  Z = diag(1, 1, sign(det(U V^T)));  R = V Z U^T;  s = trace(R C) / var;  t = mu_q - s R mu_p
+ *   PA = (1/N) sum_i |s R p_i + t - q_i|        RA = (1/N) sum_i |(p_i - r_p) - (q_i - r_q)|
+ * A hand whose var is exactly 0 (e.g. all predicted points equal, or N = 1) is degenerate.
+ * pred, gt (B,N,3), N >= 1; root_pred, root_gt (B,3) or NULL (= point 0); hand_valid (B) or NULL (0 = invalid, else valid).
+ * per_hand (B,2) or NULL: [PA, RA] per hand, NaN where hand_valid == 0, PA NaN where degenerate.
+ * aligned (B,N,3) or NULL: s R p + t for every hand, NaN where degenerate.   partial: (B, HB_KP_SUMS) scratch.
+ * sums: [0] sum of PA over valid non-degenerate hands, [1] their count,
+ *       [2] sum of RA over valid hands, [3] their count, [4] valid hands excluded as degenerate, [5..7] 0.
+ * Fixed reduction order: bit-reproducible, ready for a packed all-reduce.  No gradient. */
+int hb_procrustes_metrics(const float* pred, const float* gt, int B, int N, const float* root_pred,
+                          const float* root_gt, const float* hand_valid, float* per_hand, float* aligned,
+                          float* partial, float* sums, void* stream);
 /* GT-side glue of process_data_light (src/callbacks/process/process_arctic.py:42-65), one hand side, after the no-grad MANO
  * forward of the ground-truth parameters (hb_mano_head_fwd with HB_POSE_AXIS_ANGLE, cam = K = NULL):
  *   Tr0 = mean_j (j3d_full - joints3d);  v3d_cam = vertices + Tr0;  cam_t = j3d_full[:,0] - joints3d[:,0];
