@@ -288,14 +288,27 @@ class RotApplyFunction(torch.autograd.Function):
         return None, gm
 
 
+CROP_DTYPES = (torch.float32, torch.bfloat16)
+
+
+def check_crop_dtype(dtype):
+    """The crop layer writes fp32 or bf16 crop planes (hb_pcl_fwd*, hb_pcl_fwd*_bf16); anything else is an error."""
+    if dtype not in CROP_DTYPES:
+        raise TypeError(f"out_dtype: expected torch.float32 or torch.bfloat16, got {dtype}")
+    return dtype
+
+
 class PerspectiveCropFunction(torch.autograd.Function):
     """Batched Perspective Crop Layer (src/datasets/hands_light_dataset.py:354-467).
     img (Bi,C,R,R); bbox (Bi*n,4) int32; K (Bi*n,3,3) -> crop (Bi*n,C,R,R), R_virt2orig (Bi*n,3,3).
-    Gradient w.r.t. img only (the sampling grid is data)."""
+    Gradient w.r.t. img only (the sampling grid is data).
+    out_dtype torch.bfloat16: the crop is written as bf16 (the RNE rounding of the fp32 crop) and its gradient is read as
+    bf16; R_virt2orig and the image gradient stay fp32."""
 
     @staticmethod
-    def forward(ctx, img, bbox, K, crops_per_img, mean=None, std=None):
+    def forward(ctx, img, bbox, K, crops_per_img, mean=None, std=None, out_dtype=torch.float32):
         lib = _lib.load()
+        bf16 = check_crop_dtype(out_dtype) == torch.bfloat16
         needs_grad = bool(img.requires_grad)   # read before _f32c: .contiguous() of a strided image is a new tensor
         u8 = isinstance(img, torch.Tensor) and img.dtype == torch.uint8
         if u8:
@@ -333,18 +346,21 @@ class PerspectiveCropFunction(torch.autograd.Function):
         K = _f32c(K.to(dev) if isinstance(K, torch.Tensor) else K, "K", (n, 3, 3))
         params = torch.empty(n, _lib.PCL_PARAM_FLOATS, dtype=torch.float32, device=dev)
         rot = torch.empty(n, 3, 3, dtype=torch.float32, device=dev)
-        out = torch.empty(n, C, R, R, dtype=torch.float32, device=dev)
+        out = torch.empty(n, C, R, R, dtype=out_dtype, device=dev)
         with torch.cuda.device(dev):
             _lib.check(lib.hb_pcl_setup(_ptr(bbox), _ptr(K), n, R, _ptr(params), _ptr(rot), _stream()), "hb_pcl_setup")
             if u8:
                 m = (ctypes.c_float * C)(*[float(v) for v in mean])
                 sd = (ctypes.c_float * C)(*[float(v) for v in std])
-                _lib.check(lib.hb_pcl_fwd_u8(_ptr(img), ctypes.cast(m, ctypes.c_void_p), ctypes.cast(sd, ctypes.c_void_p), _ptr(params), n,
-                                             crops_per_img, C, R, _ptr(out), _stream()), "hb_pcl_fwd_u8")
+                name = "hb_pcl_fwd_u8_bf16" if bf16 else "hb_pcl_fwd_u8"
+                _lib.check(getattr(lib, name)(_ptr(img), ctypes.cast(m, ctypes.c_void_p), ctypes.cast(sd, ctypes.c_void_p), _ptr(params), n,
+                                              crops_per_img, C, R, _ptr(out), _stream()), name)
             else:
-                _lib.check(lib.hb_pcl_fwd(_ptr(img), _ptr(params), n, crops_per_img, C, R, _ptr(out), _stream()), "hb_pcl_fwd")
+                name = "hb_pcl_fwd_bf16" if bf16 else "hb_pcl_fwd"
+                _lib.check(getattr(lib, name)(_ptr(img), _ptr(params), n, crops_per_img, C, R, _ptr(out), _stream()), name)
         ctx.save_for_backward(params)
         ctx.dims = (Bi, C, R, crops_per_img)
+        ctx.bf16 = bf16
         ctx.mark_non_differentiable(rot)
         return out, rot
 
@@ -355,13 +371,15 @@ class PerspectiveCropFunction(torch.autograd.Function):
         Bi, C, R, cpi = ctx.dims
         n = Bi * cpi
         dev = params.device
-        g_out = g_out.contiguous().float()
+        # a bf16 crop takes its gradient as bf16 (what the consumer's backward produces under autocast), read by the kernel as is
+        g_dtype, name = (torch.bfloat16, "hb_pcl_bwd_bf16") if ctx.bf16 else (torch.float32, "hb_pcl_bwd")
+        g_out = g_out.contiguous().to(g_dtype)
         g_img = torch.empty(Bi, C, R, R, dtype=torch.float32, device=dev)
         nbytes = lib.hb_pcl_bwd_workspace_bytes(n, cpi, C, R)
         ws = _workspace(nbytes, dev)
         with torch.cuda.device(dev):
-            _lib.check(lib.hb_pcl_bwd(_ptr(g_out), _ptr(params), n, cpi, C, R, _ptr(g_img), _ptr(ws), nbytes, _stream()), "hb_pcl_bwd")
-        return g_img, None, None, None, None, None
+            _lib.check(getattr(lib, name)(_ptr(g_out), _ptr(params), n, cpi, C, R, _ptr(g_img), _ptr(ws), nbytes, _stream()), name)
+        return g_img, None, None, None, None, None, None
 
 
 class SilhouetteHandle:

@@ -3,10 +3,10 @@ reference, where the closure at src/datasets/hands_light_dataset.py:354-467 runs
 CPU inside the data loader)."""
 import torch
 
-from .functional import PerspectiveCropFunction, RotApplyFunction
+from .functional import PerspectiveCropFunction, RotApplyFunction, check_crop_dtype
 
 
-def perspective_crop(img, bbox_xyxy, K, img_res=224, crops_per_img=1, mean=None, std=None):
+def perspective_crop(img, bbox_xyxy, K, img_res=224, crops_per_img=1, mean=None, std=None, out_dtype=torch.float32):
     """img (Bi,3,img_res,img_res) fp32 CUDA; bbox_xyxy (Bi*crops_per_img,4) int [x0,y0,x1,y1] inside the
     image; K (Bi*crops_per_img,3,3).  Crop c samples image c // crops_per_img.
     Returns crop (Bi*crops_per_img,3,img_res,img_res) and R_virt2orig (Bi*crops_per_img,3,3).
@@ -14,10 +14,15 @@ def perspective_crop(img, bbox_xyxy, K, img_res=224, crops_per_img=1, mean=None,
 
     Extension: `img` may be the data loader's uint8 image with `mean`/`std` (the reference's img_norm_mean/std, C floats):
     the normalisation (u/255 - mean)/std the reference applies before the crop (hands_light_dataset.py:177-184) is fused
-    into the gather -- same crops, a quarter of the bytes over PCIe.  No gradient flows to a uint8 image."""
+    into the gather -- same crops, a quarter of the bytes over PCIe.  No gradient flows to a uint8 image.
+
+    out_dtype=torch.bfloat16 (for a backbone trained under bf16 autocast): the crop is returned as bf16, bit-identical to
+    the fp32 crop rounded to nearest even, and its gradient is consumed as bf16 -- no cast kernel on either side.
+    R_virt2orig and the gradient w.r.t. an fp32 `img` stay fp32.  Any other dtype raises TypeError."""
+    check_crop_dtype(out_dtype)
     if img.shape[-1] != img_res or img.shape[-2] != img_res:
         raise ValueError(f"img must be {img_res}x{img_res} (the reference crops from the resized full image)")
-    return PerspectiveCropFunction.apply(img, bbox_xyxy, K, int(crops_per_img), mean, std)
+    return PerspectiveCropFunction.apply(img, bbox_xyxy, K, int(crops_per_img), mean, std, out_dtype)
 
 
 def apply_virtual_rotation(R_virt2orig, pose):

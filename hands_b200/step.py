@@ -16,7 +16,7 @@ import ctypes
 import torch
 
 from . import _lib
-from .functional import ManoHandle, _ptr
+from .functional import ManoHandle, _ptr, check_crop_dtype
 from .synthetic import synthetic_head_inputs, synthetic_mano_buffers, synthetic_pcl_inputs
 
 NV, NJ, NOJ, NB = 778, 16, 21, 10
@@ -27,8 +27,12 @@ class GeometryStep:
     IMG_STD = (0.229, 0.224, 0.225)
 
     def __init__(self, samples, device, img_res=224, with_pcl=True, with_mano=True, hands_per_sample=2, seed=0, grads_on=("v3d", "j3d", "j2d"),
-                 src_u8=False):
+                 src_u8=False, crop_dtype=torch.float32):
+        """crop_dtype torch.bfloat16: `crops` and `g_crops` are bf16 (what a backbone under bf16 autocast reads and returns) and
+        the step runs the bf16 crop-layer entry points; the image, its gradient and everything MANO stay fp32."""
         self.lib = _lib.load()
+        self.crop_dtype = check_crop_dtype(crop_dtype)
+        self.crop_bf16 = crop_dtype == torch.bfloat16
         self.S, self.dev, self.R = int(samples), torch.device(device), int(img_res)
         self.with_pcl, self.with_mano, self.hps = with_pcl, with_mano, hands_per_sample
         self.grads_on = grads_on
@@ -48,8 +52,9 @@ class GeometryStep:
                 self._std = (ctypes.c_float * 3)(*self.IMG_STD)
             else:
                 self.img = torch.randn(S, 3, R, R, generator=gen, **f32)
-            self.crops = torch.empty(n, 3, R, R, **f32)
-            self.g_crops = torch.randn(n, 3, R, R, generator=gen, **f32)
+            self.crops = torch.empty(n, 3, R, R, dtype=crop_dtype, device=dev)
+            # drawn in fp32 either way, so the generator's later draws (the MANO gradients) do not depend on crop_dtype
+            self.g_crops = torch.randn(n, 3, R, R, generator=gen, **f32).to(crop_dtype)
             self.g_img = torch.empty(S, 3, R, R, **f32)
             self.params = torch.empty(n, _lib.PCL_PARAM_FLOATS, **f32)
             self.rot = torch.empty(n, 3, 3, **f32)
@@ -94,18 +99,24 @@ class GeometryStep:
         _lib.check(self.lib.hb_pcl_setup(_ptr(self.bbox), _ptr(self.Kcrop), self.n, self.R, _ptr(self.params), _ptr(self.rot), self._st()), "hb_pcl_setup")
 
     def pcl_forward(self):
+        sfx = "_bf16" if self.crop_bf16 else ""
         if self.src_u8:
-            _lib.check(self.lib.hb_pcl_fwd_u8(_ptr(self.img), ctypes.cast(self._mean, ctypes.c_void_p), ctypes.cast(self._std, ctypes.c_void_p), _ptr(self.params),
-                                              self.n, self.hps, 3, self.R, _ptr(self.crops), self._st()), "hb_pcl_fwd_u8")
+            fn = "hb_pcl_fwd_u8" + sfx
+            _lib.check(getattr(self.lib, fn)(_ptr(self.img), ctypes.cast(self._mean, ctypes.c_void_p), ctypes.cast(self._std, ctypes.c_void_p), _ptr(self.params),
+                                             self.n, self.hps, 3, self.R, _ptr(self.crops), self._st()), fn)
             return
-        _lib.check(self.lib.hb_pcl_fwd(_ptr(self.img), _ptr(self.params), self.n, self.hps, 3, self.R, _ptr(self.crops), self._st()), "hb_pcl_fwd")
+        fn = "hb_pcl_fwd" + sfx
+        _lib.check(getattr(self.lib, fn)(_ptr(self.img), _ptr(self.params), self.n, self.hps, 3, self.R, _ptr(self.crops), self._st()), fn)
 
     def pcl_backward(self):
-        _lib.check(self.lib.hb_pcl_bwd(_ptr(self.g_crops), _ptr(self.params), self.n, self.hps, 3, self.R, _ptr(self.g_img), _ptr(self.pcl_ws),
-                                       self.pcl_ws_bytes, self._st()), "hb_pcl_bwd")
+        fn = "hb_pcl_bwd_bf16" if self.crop_bf16 else "hb_pcl_bwd"
+        _lib.check(getattr(self.lib, fn)(_ptr(self.g_crops), _ptr(self.params), self.n, self.hps, 3, self.R, _ptr(self.g_img), _ptr(self.pcl_ws),
+                                         self.pcl_ws_bytes, self._st()), fn)
 
     def pcl_backward_stage(self, stages):
         """stages 1 = transposed resize, 2 = transposed gather (single-chunk batches only; used by bench.py's roofline leg)."""
+        if self.crop_bf16:
+            raise NotImplementedError("pcl_backward_stage: the stage-by-stage entry point (hb_pcl_bwd_stages) takes fp32 crop gradients only")
         _lib.check(self.lib.hb_pcl_bwd_stages(_ptr(self.g_crops), _ptr(self.params), self.n, self.hps, 3, self.R, _ptr(self.g_img), _ptr(self.pcl_ws),
                                               self.pcl_ws_bytes, int(stages), self._st()), "hb_pcl_bwd_stages")
 
@@ -193,15 +204,19 @@ class GeometryStep:
     def mano_bytes_per_hand(self):
         return 31068.0
 
+    def crop_elem_bytes(self):
+        return 2 if self.crop_bf16 else 4
+
     def pcl_bytes_per_crop(self):
-        return 3 * self.R * self.R * 4 * 3 + 12.0 * self.mean_s2  # out write + g_out read + g_img write + src footprint
+        # out write + g_out read (crop dtype) + g_img write (fp32) + src footprint
+        return 3 * self.R * self.R * (2 * self.crop_elem_bytes() + 4) + 12.0 * self.mean_s2
 
     def bytes_per_sample(self):
         b = 0.0
         if self.with_mano:
             b += self.hps * self.mano_bytes_per_hand()
         if self.with_pcl:
-            plane = 3 * self.R * self.R * 4
+            plane = 3 * self.R * self.R * self.crop_elem_bytes()   # the crop and its gradient, in the crop dtype
             # SURVEY.md §8(d) convention for crops sharing one source image: 2*hps planes + the source footprints
             # (4 x 602,112 + 2 x 12 s^2 for two hands; the shared g_img write is not counted, so the figure is
             # conservative -- real traffic is one plane higher)

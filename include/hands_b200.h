@@ -10,8 +10,9 @@
  * Conventions
  *   - every function returns int: 0 = OK, <0 = argument error (HB_E_*), >0 = cudaError_t.
  *     hb_last_error_string() gives the text of the last failure on the calling thread.
- *   - all tensors are fp32, contiguous, row-major; pointers are DEVICE pointers unless the
- *     parameter name ends in _host.  Float buffers must be 8-byte aligned.
+ *   - all tensors are fp32, contiguous, row-major (except the bf16 crop planes of the *_bf16 crop-layer
+ *     entry points); pointers are DEVICE pointers unless the parameter name ends in _host.  Float buffers
+ *     must be 8-byte aligned.
  *   - the caller allocates and owns every buffer, including the workspace; the library never
  *     allocates per call and never frees caller memory.
  *   - `stream` is a cudaStream_t passed as void*; launches are asynchronous on it.
@@ -53,7 +54,7 @@ typedef struct hb_mano hb_mano; /* opaque: MANO constants of one hand side on on
 #define HB_ROT6D_COLS 1        /* src/models/hamer_light/geometry.py:47-62, src/models/handoccnet_light/mano_head.py:132-141: a1=x[0:3], a2=x[3:6], COLUMNS */
 #define HB_ROT6D_COLS_PAIRED 2 /* common/rot.py:367-381: a1=x[0,2,4], a2=x[1,3,5], COLUMNS */
 
-#define HB_VERSION 205 /* hb_version() of a matching binary */
+#define HB_VERSION 206 /* hb_version() of a matching binary */
 const char* hb_last_error_string(void);
 int hb_version(void);
 
@@ -256,6 +257,24 @@ int hb_pcl_bwd(const float* g_out, const float* params, int n_crops, int crops_p
  * meaningful stage by stage when the whole batch fits one chunk of the workspace. */
 int hb_pcl_bwd_stages(const float* g_out, const float* params, int n_crops, int crops_per_img, int C, int img_res,
                       float* g_img, void* workspace, size_t workspace_bytes, int stages, void* stream);
+
+/* bf16 crop planes, for backbones trained under bf16 autocast: the crop is written in the dtype its consumer reads and
+ * its gradient is read in the dtype the consumer's backward produces, so no cast kernel runs on either side.
+ * bf16 buffers hold bfloat16 bit patterns (uint16_t), round-to-nearest-even; they need only 2-byte alignment (better
+ * alignment selects the vector paths, never a different result than stated below).  The source image and g_img stay fp32.
+ *   hb_pcl_fwd_bf16 / hb_pcl_fwd_u8_bf16: `out` (n_crops,C,R,R) bf16 is bit-identical to the RNE bf16 rounding of what
+ *     hb_pcl_fwd / hb_pcl_fwd_u8 write for the same inputs in the same arithmetic mode (hb_pcl_set_exact), i.e.
+ *     crop_fp32.to(torch.bfloat16).  All internal arithmetic is fp32; only the final store rounds.
+ *   hb_pcl_bwd_bf16: `g_img` (fp32) is bit-identical to hb_pcl_bwd on the exactly widened gradient g_out.float(), for the
+ *     same workspace size (hence the same chunking) and g_out buffers aligned alike in elements.  Widening is exact, so
+ *     the arithmetic and its order are those of hb_pcl_bwd.  hb_pcl_bwd_workspace_bytes serves both.
+ * Argument errors are those of the fp32 twins (HB_E_ARG, HB_E_WORKSPACE, HB_E_ALIGN), with messages naming the function. */
+int hb_pcl_fwd_bf16(const float* img, const float* params, int n_crops, int crops_per_img, int C, int img_res,
+                    uint16_t* out, void* stream);
+int hb_pcl_fwd_u8_bf16(const uint8_t* img, const float* mean_host, const float* std_host, const float* params,
+                       int n_crops, int crops_per_img, int C, int img_res, uint16_t* out, void* stream);
+int hb_pcl_bwd_bf16(const uint16_t* g_out, const float* params, int n_crops, int crops_per_img, int C, int img_res,
+                    float* g_img, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- soft silhouette of the hand mesh -----------------------------------------------------------
  * Replaces: src/models/hands_light/renderer.py:124-199 (pytorch3d MeshRasterizer + SoftSilhouetteShader as configured at
