@@ -266,7 +266,9 @@ def persp_to_weak(cam_t, focal, img_res):
 
 
 class RotApplyFunction(torch.autograd.Function):
-    """out[b] = R[b] @ M[b]  (src/models/hands_light/model.py:330-334); gradient to M only (R is data)."""
+    """out[b] = R[b] @ M[b]  (src/models/hands_light/model.py:330-334).  Gradients: g_M = R^T g, and g_R = g M^T when R
+    requires grad (the crop layer's R_virt2orig does not; a `pre_rot` that is itself a prediction does, and the reference's
+    torch product would give it this gradient through the returned `pose`)."""
 
     @staticmethod
     def forward(ctx, R, M):
@@ -275,17 +277,26 @@ class RotApplyFunction(torch.autograd.Function):
         out = torch.empty_like(M)
         with torch.cuda.device(M.device):
             _lib.check(_lib.load().hb_rot_apply(_ptr(R), _ptr(M), M.shape[0], 0, _ptr(out), _stream()), "hb_rot_apply")
-        ctx.save_for_backward(R)
+        ctx.save_for_backward(R, M if ctx.needs_input_grad[0] else None)
         return out
 
     @staticmethod
     def backward(ctx, g):
-        (R,) = ctx.saved_tensors
+        R, M = ctx.saved_tensors
         g = g.contiguous().float()
-        gm = torch.empty_like(g)
+        gr = gm = None
+        lib = _lib.load()
         with torch.cuda.device(g.device):
-            _lib.check(_lib.load().hb_rot_apply(_ptr(R), _ptr(g), g.shape[0], 1, _ptr(gm), _stream()), "hb_rot_apply")
-        return None, gm
+            if ctx.needs_input_grad[0]:
+                gr = torch.empty_like(g)
+                # g M^T = (M g^T)^T: the same kernel on transposed operands
+                gt = g.transpose(1, 2).contiguous()
+                _lib.check(lib.hb_rot_apply(_ptr(M), _ptr(gt), g.shape[0], 0, _ptr(gr), _stream()), "hb_rot_apply")
+                gr = gr.transpose(1, 2)
+            if ctx.needs_input_grad[1]:
+                gm = torch.empty_like(g)
+                _lib.check(lib.hb_rot_apply(_ptr(R), _ptr(g), g.shape[0], 1, _ptr(gm), _stream()), "hb_rot_apply")
+        return gr, gm
 
 
 CROP_DTYPES = (torch.float32, torch.bfloat16)

@@ -32,7 +32,8 @@ class MANOHead(nn.Module):
         rotmat: (B,16,3,3) rotation matrices, or (B,48) axis-angle
         shape:  (B,10) betas;  cam: (B,3) weak-perspective [s,tx,ty];  K: (B,3,3) intrinsics
         pre_rot (extension, default None): (B,3,3) R_virt2orig fused onto the global orientation
-                (the PCL fix-up of hands_light/model.py:330-334) instead of a separate in-place bmm.
+                (the PCL fix-up of hands_light/model.py:330-334) instead of a separate in-place bmm.  A pre_rot
+                that requires grad receives it through every output, the returned `pose` included.
         """
         pose = rotmat if rotmat.shape[-1] == 48 else rotmat.reshape(-1, 16, 3, 3)
         if pre_rot is not None:
